@@ -2,6 +2,7 @@
 """Benchmark of the sparse-vae hot path on B200: TransformerVAE training tokens/sec at seq 4096.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c4|c5] [--kernel-only]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "C2"): TransformerVAE with the default hparams dataclass (d_model 512, 8 heads,
 6 decoder layers + Perceiver encoder, block-sparse attention window 4, latent 64, tied 32768-token embedding,
@@ -24,6 +25,12 @@ One JSON line on stdout (rank 0):
 `sample(4096, 256)` through the graphed decoder + one chunked teacher-forced reconstruct; its own metric).
 `--impl reference` times that CPU restatement alone (the reference itself is Python/Triton-1.1 and cannot run on
 this box; see DESIGN.md).  `--kernel-only` runs just the attention kernels at the C2 shape (short; for ncu).
+`--steps K` is the number of timed steps of every mode; without it, 50 (training, --kernel-only) or 5 (c5 and
+--impl reference, whose steps take seconds).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last of them computed as .npy files -- for
+training (c2 / c4) the loss and the parameters and gradients it left in the model (see `dump_outputs`), for c5 the
+sampled token ids.  Model init, token batches and random streams are seeded, so two builds run with the same arguments
+can be compared file by file.
 """
 from __future__ import annotations
 
@@ -54,7 +61,8 @@ WINDOW = 4            # TransformerVAEHparams().sparse_self_attention window (Sp
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=50)
+    ap.add_argument('--steps', type=int, default=None,
+                    help='timed steps (default 50; 5 for --config c5 and --impl reference)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='c2', choices=['c2', 'c4', 'c5'],
@@ -68,7 +76,17 @@ def parse():
     ap.add_argument('--kernel-only', action='store_true')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--cpu-sample-seqs', type=int, default=1)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/<name>.npy (training: loss, parameters and '
+                         'gradients; c5: the sampled token ids)')
     args = ap.parse_args()
+    slow_steps = args.impl == 'reference' or args.config == 'c5'
+    args.steps = (5 if slow_steps else 50) if args.steps is None else args.steps
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl == 'reference' or (args.kernel_only and args.config != 'c5')):
+        ap.error('--dump-outputs applies to the training step (c2, c4) and to generation (c5) of --impl ours, '
+                 'not to --kernel-only')
     shape = {'c2': (BATCH_PER_GPU, SEQ), 'c4': (4, 16384), 'c5': (256, 4096)}[args.config]
     args.batch = shape[0] if args.batch is None else args.batch
     args.seq = shape[1] if args.seq is None else args.seq
@@ -187,7 +205,7 @@ def main_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 5)), max(0, min(args.warmup, 1))
+    steps, warmup = args.steps, max(0, min(args.warmup, 1))
     if args.config == 'c5':
         res = run_cpu_decoder_forward(args, steps, warmup)
         cfg = generation_config(args, 1)
@@ -429,6 +447,29 @@ def bottleneck_leg(dev):
 
 
 # ------------------------------------------------------------------------------------------ our arm
+DUMP_SAMPLE = 65536
+
+
+def dump_outputs(out_dir: str, loss: torch.Tensor, model: torch.nn.Module):
+    """Writes what the caller of a training step gets from it, as float32: `loss.npy`, and for every parameter
+    `param.<name>.npy` (its value after the optimizer step) and `grad.<name>.npy` (the clipped gradient the step applied).
+    A tensor of more than DUMP_SAMPLE elements is stored as DUMP_SAMPLE elements at flat positions drawn with
+    numpy's default_rng(7295), the same positions in every run; the default model comes to about 35 MiB."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / 'loss.npy', loss.detach().float().cpu().numpy())
+    for name, p in model.named_parameters():
+        idx = None
+        if p.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(7295).choice(p.numel(), DUMP_SAMPLE, replace=False))
+            idx = torch.from_numpy(idx).to(p.device)
+        for kind, t in (('param', p), ('grad', p.grad)):
+            if t is not None:
+                t = t.detach() if idx is None else t.detach().reshape(-1)[idx]
+                np.save(out / f'{kind}.{name}.npy', t.float().cpu().numpy())
+
+
 def main_ours(args):
     import torch.distributed as dist
     import sparse_vae_b200 as sv
@@ -497,11 +538,18 @@ def main_ours(args):
             step(resident[i % n_host])
 
     # ---- device-resident inputs: the headline `value`
+    last_loss = [None]
+
+    def headline_step(i):
+        last_loss[0] = step(resident[i % n_host])
+
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms = timed(lambda i: step(resident[i % n_host]), args.steps)
+    ms = timed(headline_step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss[0], model)
     tokens = world * B * L * args.steps
     value = tokens / (ms * 1e-3)
 
@@ -644,14 +692,24 @@ def main_generation(args):
         rec_ms, _ = timed(reconstruct_all, 2)
         rec = {'what': f'teacher-forced decoder forward + argmax, {B} x {L} tokens in chunks of 32, bf16', 'ms': rec_ms / 2,
                'tokens_per_s': world * B * L / (rec_ms / 2 * 1e-3)}
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 3))     # one step = 4095 graph replays (~1.7 s)
+    steps, warmup = args.steps, max(1, min(args.warmup, 3))      # one step = 4095 graph replays (~1.7 s)
     for i in range(warmup):
         sample(i)
+    last_ids = [None]
+
+    def headline_sample(i):
+        last_ids[0] = sample(i)
+        return last_ids[0]
+
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms, n = timed(sample, steps)
+    ms, n = timed(headline_sample, steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:               # token ids < 2 ** 24: exact in float32
+        import numpy as np
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
+        np.save(Path(args.dump_outputs) / 'token_ids.npy', last_ids[0].float().cpu().numpy())
     ms_e2e, n_e2e = timed(lambda i: sample(i, True), steps)
     N.profile_begin()
     sample(0)

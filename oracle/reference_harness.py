@@ -1,8 +1,9 @@
 """Oracle (test infrastructure): import the UNMODIFIED reference package behind import stubs.
 
-Only usable in the build container, where /root/reference exists; it is used by
-tests/golden/make_golden.py to generate the committed golden fixtures and by the optional
-`reference`-marked CPU tests.  Nothing that runs on the GPU box imports this module.
+Only usable where the environment variable SPARSE_VAE_REFERENCE names a checkout of
+norabelrose/sparse-vae; it is used by tests/golden/make_golden.py to generate the committed golden
+fixtures and by the optional `reference`-marked CPU tests, which skip without it.  The product code
+never imports this module.
 
 Why stubs are needed (SURVEY.md §0, §8c): the reference at HEAD imports two files that are missing
 from its tree (core/activation_offload.py, core/rotary_embedding.py), depends on packages that are
@@ -15,6 +16,7 @@ from __future__ import annotations
 
 import contextlib
 import importlib
+import os
 import sys
 import types
 from pathlib import Path
@@ -22,11 +24,21 @@ from pathlib import Path
 import torch
 from torch import nn
 
-REFERENCE_ROOT = Path('/root/reference')
+REFERENCE_ROOT = Path(os.environ['SPARSE_VAE_REFERENCE']) if os.environ.get('SPARSE_VAE_REFERENCE') else None
 
 
 def available() -> bool:
-    return (REFERENCE_ROOT / 'sparse_vae' / 'core' / 'sparse_attention.py').exists()
+    try:
+        return REFERENCE_ROOT is not None and (REFERENCE_ROOT / 'sparse_vae' / 'core' / 'sparse_attention.py').exists()
+    except OSError:                      # a path this user may not traverse counts as absent
+        return False
+
+
+def require_reference() -> Path:
+    """REFERENCE_ROOT, or a RuntimeError saying how to name the checkout."""
+    if not available():
+        raise RuntimeError("SPARSE_VAE_REFERENCE does not name a checkout of norabelrose/sparse-vae")
+    return REFERENCE_ROOT
 
 
 class AttributeDict(dict):
@@ -124,17 +136,16 @@ _ref = None
 
 
 def load_reference():
-    """Returns the imported reference `sparse_vae` package (modules executed from /root/reference)."""
+    """Returns the imported reference `sparse_vae` package (modules executed from REFERENCE_ROOT)."""
     global _ref
     if _ref is not None:
         return _ref
-    if not available():
-        raise RuntimeError("/root/reference is not present (it only exists in the build container)")
+    root = require_reference()
     install_stubs()
     # `sparse_vae/__init__.py` star-imports data modules needing network-era packages; import the
     # sub-packages we need directly from a namespace so that the unmodified source files execute.
     pkg = types.ModuleType('sparse_vae')
-    pkg.__path__ = [str(REFERENCE_ROOT / 'sparse_vae')]
+    pkg.__path__ = [str(root / 'sparse_vae')]
     sys.modules['sparse_vae'] = pkg
     core = importlib.import_module('sparse_vae.core')
     tv = importlib.import_module('sparse_vae.transformer_vae')

@@ -1,6 +1,6 @@
 """Running the reference's own scripts, UNCHANGED, against this package.
 
-    python -m sparse_vae_b200.compat /root/reference/train.py transformer-vae trainer.max_steps=20 ...
+    python -m sparse_vae_b200.compat <norabelrose/sparse-vae checkout>/train.py transformer-vae trainer.max_steps=20 ...
 
 The reference's `train.py` / `sample.py` / `reconstruct.py` import `sparse_vae`, `pytorch_lightning` and `omegaconf`
 (train.py:1-9, sample.py:1, reconstruct.py:1-2).  This image has neither Lightning nor OmegaConf and no network for

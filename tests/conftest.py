@@ -13,18 +13,19 @@ GOLDEN = ROOT / 'tests' / 'golden'
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (B200); run with -m gpu on the GPU box')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (build container only)')
+    config.addinivalue_line('markers', 'reference: needs a checkout of norabelrose/sparse-vae named by SPARSE_VAE_REFERENCE')
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
+    from oracle import reference_harness
     has_gpu = torch.cuda.is_available()
-    has_ref = Path('/root/reference/sparse_vae').exists()
+    has_ref = reference_harness.available()
     for item in items:
         if 'gpu' in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason='no CUDA device'))
         if 'reference' in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason='/root/reference not present'))
+            item.add_marker(pytest.mark.skip(reason='SPARSE_VAE_REFERENCE does not name a checkout of norabelrose/sparse-vae'))
 
 
 @pytest.fixture(scope='session')

@@ -1,8 +1,8 @@
 """Generates the golden fixtures in this directory by running the UNMODIFIED reference
-(/root/reference, imported behind the stubs of oracle/reference_harness.py) on CPU in fp32.
+(a checkout of norabelrose/sparse-vae, imported behind the stubs of oracle/reference_harness.py) on CPU in fp32.
 
-Run in the build container only:   python tests/golden/make_golden.py
-The fixtures are committed; tests read the .npz files and never touch /root/reference.
+Run with that checkout named:   SPARSE_VAE_REFERENCE=<checkout> python tests/golden/make_golden.py
+The fixtures are committed; tests read the .npz files and never touch the reference.
 
 Inputs are produced with numpy's legacy `RandomState` (bit-stable across numpy versions) so that only
 the reference's OUTPUTS need to be stored.  Seed 7295 is the reference's own (train.py:15).
@@ -114,6 +114,13 @@ def gen_layouts(ref):
                         big=np.asarray(big, dtype=object).astype(str), **packed)
 
 
+def attention_rows(case):
+    """The sequence positions whose rows of out / dq / dk / dv are stored: a seeded three quarters of them, which keeps
+    attention_golden.npz under 1 MB."""
+    L = case['L']
+    return np.sort(np.random.RandomState(case['seed']).choice(L, 3 * L // 4, replace=False))
+
+
 def gen_attention(ref):
     SA = ref.core.SparseAttention
     store = {}
@@ -125,8 +132,10 @@ def gen_attention(ref):
         kpm = torch.tensor(pad) * -1e7 if pad is not None else None        # core/attention.py:79
         out = sa(qt, kt, vt, key_padding_mask=kpm)                          # the reference's own __call__
         out.backward(torch.tensor(dout))
+        rows = attention_rows(case)
+        store[f"{case['name']}.rows"] = rows
         for nm, t in (('out', out), ('dq', qt.grad), ('dk', kt.grad), ('dv', vt.grad)):
-            store[f"{case['name']}.{nm}"] = t.detach().numpy().astype(np.float32)
+            store[f"{case['name']}.{nm}"] = t.detach().numpy().astype(np.float32)[:, :, rows]
     np.savez_compressed(OUT / 'attention_golden.npz', **store)
 
 

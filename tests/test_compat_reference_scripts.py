@@ -1,6 +1,7 @@
 """The reference's own scripts run UNCHANGED against this package through `python -m sparse_vae_b200.compat <script>`
 (north star: "train.py, sample.py and reconstruct.py run unchanged against it").  CPU: the dense transformer-lm (the
-sparse kernels are CUDA-only); needs /root/reference, so these run in the build container only."""
+sparse kernels are CUDA-only); the two tests that run the scripts need a checkout of norabelrose/sparse-vae named by the
+environment variable SPARSE_VAE_REFERENCE and skip without one."""
 import os
 import subprocess
 import sys
@@ -8,8 +9,9 @@ from pathlib import Path
 
 import pytest
 
+from oracle.reference_harness import REFERENCE_ROOT as REF
+
 ROOT = Path(__file__).resolve().parents[1]
-REF = Path('/root/reference')
 TINY = ['model.d_model=64', 'model.num_layers=2', 'model.num_heads=2', 'model.sparse_self_attention=false',
         'data.tokens_per_batch=512', 'data.seq_len=128', 'trainer.accumulate_grad_batches=1', 'trainer.precision=32',
         'trainer.log_every_n_steps=1']

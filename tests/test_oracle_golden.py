@@ -61,18 +61,24 @@ def test_attention_oracle_matches_reference(case, golden_dir):
     out = oattn.dense_masked_attention(qt, kt, vt, lay, 32, case['causal'], kpm)
     out.backward(torch.tensor(dout))
     name = case['name']
-    np.testing.assert_allclose(out.detach().numpy(), g[f'{name}.out'], rtol=1e-5, atol=2e-6)
-    np.testing.assert_allclose(qt.grad.numpy(), g[f'{name}.dq'], rtol=1e-4, atol=5e-6)
-    np.testing.assert_allclose(kt.grad.numpy(), g[f'{name}.dk'], rtol=1e-4, atol=5e-6)
-    np.testing.assert_allclose(vt.grad.numpy(), g[f'{name}.dv'], rtol=1e-4, atol=5e-6)
+    rows = g[f'{name}.rows']                            # the fixture stores these sequence positions only
+    np.testing.assert_allclose(out.detach().numpy()[:, :, rows], g[f'{name}.out'], rtol=1e-5, atol=2e-6)
+    np.testing.assert_allclose(qt.grad.numpy()[:, :, rows], g[f'{name}.dq'], rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(kt.grad.numpy()[:, :, rows], g[f'{name}.dk'], rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(vt.grad.numpy()[:, :, rows], g[f'{name}.dv'], rtol=1e-4, atol=5e-6)
     # the literal sdd->softmax->dsd restatement and the explicit backward agree with the dense form
     with torch.no_grad():
         lit = oattn.blocksparse_attention(qt, kt, vt, lay, 32, case['causal'], kpm)
         dq, dk, dv = oattn.attention_backward(qt, kt, vt, torch.tensor(dout), lay, 32, case['causal'], kpm)
-    np.testing.assert_allclose(lit.numpy(), g[f'{name}.out'], rtol=1e-5, atol=2e-6)
-    np.testing.assert_allclose(dq.numpy(), g[f'{name}.dq'], rtol=1e-4, atol=5e-6)
-    np.testing.assert_allclose(dk.numpy(), g[f'{name}.dk'], rtol=1e-4, atol=5e-6)
-    np.testing.assert_allclose(dv.numpy(), g[f'{name}.dv'], rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(lit.numpy()[:, :, rows], g[f'{name}.out'], rtol=1e-5, atol=2e-6)
+    np.testing.assert_allclose(dq.numpy()[:, :, rows], g[f'{name}.dq'], rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(dk.numpy()[:, :, rows], g[f'{name}.dk'], rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(dv.numpy()[:, :, rows], g[f'{name}.dv'], rtol=1e-4, atol=5e-6)
+    # and with each other on every position, the ones the fixture leaves out included
+    np.testing.assert_allclose(lit.numpy(), out.detach().numpy(), rtol=1e-5, atol=2e-6)
+    np.testing.assert_allclose(dq.numpy(), qt.grad.numpy(), rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(dk.numpy(), kt.grad.numpy(), rtol=1e-4, atol=5e-6)
+    np.testing.assert_allclose(dv.numpy(), vt.grad.numpy(), rtol=1e-4, atol=5e-6)
 
 
 def test_reference_kpm_is_minus_inf_in_fp16():
