@@ -252,6 +252,17 @@ SVAE_API int svae_vocab_ce_supported(int32_t vocab);
 SVAE_API int svae_vocab_ce(void* logits, int32_t dtype, int64_t rows, int32_t vocab, int64_t ld, const int64_t* labels,
                   const float* weight, float* nll, int32_t write_grad, void* stream);
 
+/* ---- per-token log-likelihood under the vocabulary head, logits never materialised (reference
+ *      core/continuous_autoencoder.py:62-88 estimate_log_prob_iw / p_of_x_given_z) ---- */
+/* h: [rows, d], w: [vocab, d], bias: [vocab] or NULL -- all `dtype` (bf16 / fp16), row strides ldh / ldw elements
+ * (multiples of 8, 16-byte aligned); vocab = 256*k, d = 64*k <= 512.  logit = round_dtype(h . w[c] + bias[c]) with fp32
+ * accumulation (what the library GEMM returns), logp[r] = logit[r, labels[r]] - logsumexp_c logit[r, c] in fp32, and
+ * logp[r] = 0 where labels[r] == 0 (column 0 still counts in the normaliser).  One tcgen05 GEMM with a running
+ * log-sum-exp in its epilogue; deterministic (fixed combination order, no atomics). */
+SVAE_API int svae_vocab_logprob_supported(int32_t vocab, int32_t d, int32_t dtype);
+SVAE_API int svae_vocab_logprob(const void* h, int64_t ldh, const void* w, int64_t ldw, const void* bias, int32_t dtype,
+                       int64_t rows, int32_t vocab, int32_t d, const int64_t* labels, float* logp, void* stream);
+
 /* ---- bias gradient of the decoder blocks' nn.Linear layers (reference core/attention.py:33-39, ------
  *      core/transformer_layer.py:20-24): out[c] = sum_r x[r, c], fp32 accumulation, deterministic two-stage sum. */
 /* x: [rows, n] (dtype), row stride ld elements, n % 8 == 0; out: fp32 [n];

@@ -47,6 +47,7 @@ EXPORTS = (
     'svae_xattn_supported', 'svae_xattn_fwd', 'svae_xattn_bwd',
     'svae_rotary_pair_workspace_floats', 'svae_rotary_pair', 'svae_embedding_bwd',
     'svae_gelu_supported', 'svae_gelu_fwd', 'svae_gelu_bwd_workspace_floats', 'svae_gelu_bwd_counters', 'svae_gelu_bwd',
+    'svae_vocab_logprob_supported', 'svae_vocab_logprob',
 )
 
 
@@ -128,6 +129,10 @@ def _load() -> C.CDLL:
     lib.svae_vocab_ce_supported.argtypes = [i32]
     lib.svae_vocab_ce.restype = C.c_int
     lib.svae_vocab_ce.argtypes = [vp, i32, i64, i32, i64, vp, vp, vp, i32, vp]
+    lib.svae_vocab_logprob_supported.restype = C.c_int
+    lib.svae_vocab_logprob_supported.argtypes = [i32, i32, i32]
+    lib.svae_vocab_logprob.restype = C.c_int
+    lib.svae_vocab_logprob.argtypes = [vp, i64, vp, i64, vp, i32, i64, i32, i32, vp, vp, vp]
     lib.svae_colsum_workspace_floats.restype = i64
     lib.svae_colsum_workspace_floats.argtypes = [i64, i32]
     lib.svae_colsum.restype = C.c_int

@@ -172,10 +172,70 @@ class Trainer:
             self.save_checkpoint(Path(self.logger.log_dir) / 'checkpoints' / f'step={self.global_step}.ckpt', model)
         return self
 
+    def test(self, model=None, test_dataloaders=None, ckpt_path=None, verbose=True, datamodule=None):
+        """Lightning 1.4 `Trainer.test`: `test_step` on every batch under `torch.no_grad()`, in eval mode and with the
+        autocast `precision` selects (as in `fit`).  Returns `[{name: value}]` with every value the model logs reduced
+        over the batches as a mean weighted by batch size; the model's training mode is restored afterwards."""
+        model = model if model is not None else getattr(self, 'model', None)
+        if model is None:
+            raise ValueError("Trainer.test needs a model")
+        device = self._device()
+        datamodule = datamodule if datamodule is not None else (self.datamodule if test_dataloaders is None else None)
+        model.trainer = self
+        if datamodule is not None:
+            datamodule.trainer = self
+            datamodule.prepare_data()
+            datamodule.setup('test')
+        if ckpt_path:
+            ckpt = torch.load(str(ckpt_path), map_location='cpu', weights_only=False)
+            model.load_state_dict(ckpt.get('state_dict', ckpt), strict=False)
+        model.to(device)
+        if hasattr(model, 'setup'):
+            model.setup('test')
+        loaders = test_dataloaders if test_dataloaders is not None else datamodule.test_dataloader()
+        if not isinstance(loaders, (list, tuple)):
+            loaders = [loaders]
+        was_training = model.training
+        model.eval()
+        ctx, _ = self._autocast(device)
+        sums, weight = {}, 0
+        try:
+            with torch.no_grad():
+                index = 0
+                for loader in loaders:
+                    for batch in loader:
+                        batch = {k: (v.to(device, non_blocking=True) if hasattr(v, 'to') else v) for k, v in batch.items()}
+                        if hasattr(model, 'logged'):
+                            model.logged.clear()
+                        with ctx:
+                            model.test_step(batch, index)
+                        n = _batch_size(batch)
+                        for k, v in getattr(model, 'logged', {}).items():
+                            v = float(v) if hasattr(v, 'item') else v
+                            if isinstance(v, (int, float)):
+                                sums[k] = sums.get(k, 0.0) + n * float(v)
+                        weight += n
+                        index += 1
+        finally:
+            model.train(was_training)
+        results = {k: v / weight for k, v in sums.items()} if weight else {}
+        self.logged_metrics = dict(results)
+        if verbose:
+            print(f"test: " + ' '.join(f"{k} {v:.4f}" for k, v in results.items()))
+        return [results]
+
     def save_checkpoint(self, path, model=None):
         path = Path(path)
         path.parent.mkdir(parents=True, exist_ok=True)
         torch.save({'state_dict': model.state_dict(), 'hyper_parameters': dict(model.hparams), 'global_step': self.global_step}, str(path))
+
+
+def _batch_size(batch) -> int:
+    for key in ('token_ids', 'num_tokens'):
+        v = batch.get(key)
+        if v is not None and hasattr(v, 'shape') and len(v.shape):
+            return int(v.shape[0])
+    return 1
 
 
 # sub-modules the reference imports by path

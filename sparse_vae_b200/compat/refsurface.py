@@ -123,13 +123,18 @@ class TextDataModule(LightningDataModule):
 
         def batches():
             for i in range(hp.num_batches):
-                host = synthetic_tokens(B, L, seed=7295 + i + (0 if split == 'train' else 10 ** 6), pin=torch.cuda.is_available())
+                offset = {'train': 0, 'heldout': 2 * 10 ** 6}.get(split, 10 ** 6)
+                host = synthetic_tokens(B, L, seed=7295 + i + offset, pin=torch.cuda.is_available())
                 host['token_ids'] = PaddedTensor.from_raw(host['token_ids'])
                 yield host
         return batches()
 
     def val_dataloader(self):
         return self.train_dataloader(split='test')
+
+    def test_dataloader(self):
+        """Held-out synthetic batches for `Trainer.test`: a seed stream disjoint from the training and validation ones."""
+        return self.train_dataloader(split='heldout')
 
 
 TextDataModuleHparams = AttrDict

@@ -153,3 +153,44 @@ def fused_vocab_nll(hidden: Tensor, linear: nn.Linear, labels: Tensor, row_chunk
     loss, _ = _VocabNLL.apply(hidden, linear.weight, linear.bias, labels_full, token_w_full, compute_dtype,
                               row_chunk or ROW_CHUNK)
     return loss
+
+
+def _eval_dtype(hidden: Tensor) -> torch.dtype:
+    return torch.get_autocast_dtype('cuda') if torch.is_autocast_enabled('cuda') else hidden.dtype
+
+
+def vocab_log_prob_supported(hidden: Tensor, linear: nn.Linear) -> bool:
+    """Can `vocab_log_prob` evaluate this head on these hidden states in the current autocast state?"""
+    dtype = _eval_dtype(hidden)
+    return bool(hidden.is_cuda and linear.weight.is_cuda and dtype in (torch.bfloat16, torch.float16)
+                and N.lib.svae_vocab_logprob_supported(linear.out_features, linear.in_features, N.svae_dtype(dtype)))
+
+
+def vocab_log_prob(hidden: Tensor, linear: nn.Linear, labels: Tensor) -> Tensor:
+    """`log_softmax(linear(hidden)[..., :-1, :])` with column 0 set to 0 afterwards, gathered at `labels` (the
+    reference's p_of_x_given_z, core/continuous_autoencoder.py:62-88), for hidden [B, L, D] and labels [B, L-1]:
+    returns [B, L-1] fp32.  Forward only; the [B, L, vocab] logits are never materialised (`svae_vocab_logprob`: one
+    GEMM whose epilogue keeps a running log-sum-exp per row).  Under 16-bit autocast the logits are rounded to that
+    dtype before the fp32 softmax, as the reference's GEMM output is."""
+    B, L, D = hidden.shape
+    if labels.shape != (B, L - 1):
+        raise ValueError(f"vocab_log_prob: labels {tuple(labels.shape)} must be the tokens shifted by one ({B}, {L - 1})")
+    if torch.is_grad_enabled() and (hidden.requires_grad or any(p.requires_grad for p in linear.parameters())):
+        raise ValueError("vocab_log_prob is forward only: call it under torch.no_grad()")
+    if not (hidden.is_cuda and linear.weight.is_cuda and labels.is_cuda):
+        raise ValueError("vocab_log_prob needs CUDA tensors")
+    dtype = _eval_dtype(hidden)
+    if not vocab_log_prob_supported(hidden, linear):
+        raise ValueError(f"vocab_log_prob: a 16-bit head with vocab = 256*k and d = 64*k <= 512 is needed "
+                         f"(got vocab {linear.out_features}, d {linear.in_features}, dtype {dtype})")
+    h = hidden.reshape(-1, D).to(dtype).contiguous()
+    w = linear.weight.to(dtype).contiguous()
+    b = linear.bias.to(dtype).contiguous() if linear.bias is not None else None
+    # the last position predicts nothing: label 0 (log-probability 0) instead of slicing the hidden states
+    lab = torch.cat([labels.long(), labels.new_zeros(B, 1, dtype=torch.long)], dim=1).reshape(-1)
+    out = torch.empty(B * L, device=hidden.device, dtype=torch.float32)
+    N.check(N.lib.svae_vocab_logprob(h.data_ptr(), h.stride(0), w.data_ptr(), w.stride(0),
+                                     b.data_ptr() if b is not None else None, N.svae_dtype(dtype), B * L,
+                                     linear.out_features, D, lab.data_ptr(), out.data_ptr(), N.current_stream(h.device)),
+            'svae_vocab_logprob')
+    return out.view(B, L)[:, :-1]

@@ -95,6 +95,26 @@ int encode_tmap(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int 
   return SVAE_OK;
 }
 
+int encode_tmap_2d(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int64_t cols, int64_t rows, int64_t ld,
+                   int box_rows) {
+  EncodeTiledFn fn = get_encode_fn();
+  SVAE_REQUIRE(fn != nullptr, SVAE_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the CUDA driver");
+  static thread_local bool context_bound = false;      // see encode_tmap
+  if (!context_bound) {
+    SVAE_CUDA_CHECK(cudaFree(nullptr));
+    context_bound = true;
+  }
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)((rows > 1 ? ld : cols) * 2)};
+  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(map, dt, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  SVAE_REQUIRE(r == CUDA_SUCCESS, SVAE_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d): base=%p dims={%lld,%lld} ld=%lld",
+               (int)r, base, (long long)cols, (long long)rows, (long long)ld);
+  return SVAE_OK;
+}
+
 }  // namespace sm100
 
 static bool tma_ok(const void* p, const int64_t s[3], int H, int B, int L) {

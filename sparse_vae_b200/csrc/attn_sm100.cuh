@@ -166,6 +166,10 @@ __device__ __forceinline__ void slot_exp_pack(const uint32_t (&v)[32], uint32_t 
 
 int encode_tmap(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int Dh, int L, int H, int B,
                 const int64_t stride[3], int box_rows);
+// 2-D map over a row-major 16-bit [rows, cols] matrix (row stride ld elements); box = 64 columns (one SWIZZLE_128B
+// row) x box_rows rows.  Rows past the end read as zeros.
+int encode_tmap_2d(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int64_t cols, int64_t rows, int64_t ld,
+                   int box_rows);
 
 }  // namespace sm100
 }  // namespace svae

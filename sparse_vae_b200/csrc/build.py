@@ -23,7 +23,7 @@ LIB = HERE / 'libsvae_b200.so'
 DEBUG_LIB = HERE / 'libsvae_b200_dbg.so'
 SOURCES = ['abi.cu', 'bottleneck.cu', 'attn_exact.cu', 'attn_fwd_sm100.cu', 'attn_fwd_persist_sm100.cu', 'attn_bwd_sm100.cu',
            'attn_bwd1_sm100.cu', 'xattn_sm100.cu', 'attn_dispatch.cu', 'optim.cu', 'layernorm.cu', 'vocab_ce.cu', 'rotary.cu', 'colsum.cu',
-           'decode_attn.cu', 'sampling.cu', 'residual.cu', 'gelu.cu', 'embedding.cu']
+           'decode_attn.cu', 'sampling.cu', 'residual.cu', 'gelu.cu', 'embedding.cu', 'vocab_ll_sm100.cu']
 DEBUG_SOURCES = ['debug_mma_bench.cu', 'debug_pipe_bench.cu'] + SOURCES       # product sources again, with -DSVAE_DEBUG_BUILD
 HEADERS = ['common.cuh', 'sm100_ptx.cuh', 'attn_sm100.cuh', '../../include/sparse_vae_b200.h',
            '../../include/sparse_vae_b200_debug.h']

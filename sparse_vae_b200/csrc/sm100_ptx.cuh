@@ -282,6 +282,14 @@ __device__ __forceinline__ void tma_load_4d_w(void* smem_dst, const CUtensorMap*
       : "memory");
 }
 
+__device__ __forceinline__ void tma_load_2d_w(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
+  asm volatile(
+      "{\n\t.reg .pred e;\n\telect.sync _|e, 0xffffffff;\n\t"
+      "@e cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];\n\t}"
+      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+      : "memory");
+}
+
 // Dependency helpers for batched tcgen05.ld: after ONE wait, tie further register arrays to it.
 __device__ __forceinline__ void tmem_dep(uint32_t (&r)[32]) {
   asm volatile("" : SVAE_DEP8(r, 0), SVAE_DEP8(r, 8) : : "memory");

@@ -4,6 +4,7 @@ position.  `training_step`, `reconstruct`, `sample`, `predict`, `test_step` keep
 logged metrics and return values; state_dict keys are identical so reference checkpoints load."""
 from __future__ import annotations
 
+import math
 from copy import deepcopy
 from dataclasses import dataclass
 from typing import Any, Dict, Optional
@@ -60,6 +61,12 @@ class TransformerVAEHparams(TransformerHparams, ContinuousVAEHparams):
 
 
 class TransformerVAE(TransformerLanguageModel, ContinuousVAE):
+    # Decoder tokens per pass of the importance-weighted estimator's fast path: latent samples are stacked along the
+    # batch so that each decoder forward covers about this many tokens (1 sample at 16 x 4096, 64 at 2 x 512).
+    IW_TOKENS_PER_PASS = 65536
+    # latent samples of test_step's importance-weighted estimate (the reference's fixed 100, one per rsample call)
+    iw_samples: int = 100
+
     # `validate_args` of the posterior `Normal` returned by `training_step`.  None = torch's default, i.e. the reference's
     # behaviour: the constructor checks loc / scale on the HOST (`constraint.check(...).all()`), which synchronises the
     # device in the middle of every step and empties the launch queue.  A trainer that wants the CPU to run ahead of the
@@ -127,11 +134,59 @@ class TransformerVAE(TransformerLanguageModel, ContinuousVAE):
         padding = original.eq(0) if padding is None else padding
         x = self.input_layer(original)
         posterior = self.q_of_z_given_x(self.encoder(x, padding=padding))
-        log_prob = self.estimate_log_prob_iw(posterior, x, original, num_samples=100, num_iter=100,
-                                             padding=padding) / batch['num_tokens']
+        log_prob = self.estimate_log_prob_iw(posterior, x, original, num_samples=self.iw_samples,
+                                             num_iter=self.iw_samples, padding=padding) / batch['num_tokens']
         nll_iw = -log_prob.mean()
         self.log('nll_iw', nll_iw, on_step=True)
         return nll_iw
+
+    def estimate_log_prob_iw(self, q_of_z: Normal, x: Tensor, labels: Tensor, num_samples: int, num_iter: int = 1,
+                             padding: Tensor = None, samples_per_pass: Optional[int] = None):
+        """Importance-weighted estimate of log p(x) per sequence (reference core/continuous_autoencoder.py:62-88).
+
+        On the GPU under 16-bit autocast, without autograd and in eval mode, the latent samples are decoded in groups
+        stacked along the batch (`samples_per_pass`, default: IW_TOKENS_PER_PASS decoder tokens per pass) and
+        log p(x|z) comes from `fused_ce.vocab_log_prob`, so the [B, L, vocab] logits and their fp32 log-softmax are never
+        allocated.  z is drawn exactly as the reference draws it (`num_iter` calls of `q_of_z.rsample([chunk])`), so
+        both forms see the same samples (eval mode is required: training-mode dropout would draw from the generator
+        between the reference's rsample calls).  Anything else runs the reference form
+        (ContinuousVAE.estimate_log_prob_iw)."""
+        head = self.output_layer[-1]
+        x_raw, _ = split_padding(x)
+        fast = (x_raw.is_cuda and torch.is_autocast_enabled('cuda') and not torch.is_grad_enabled() and not self.training
+                and torch.get_autocast_dtype('cuda') in (torch.bfloat16, torch.float16)
+                and fused_ce.vocab_log_prob_supported(x_raw, head))
+        if not fast:
+            return super().estimate_log_prob_iw(q_of_z, x, labels, num_samples, num_iter, padding)
+        assert num_samples % num_iter == 0
+        chunk = num_samples // num_iter
+        zs, log_p_z, log_q_z = [], [], []
+        for _ in range(num_iter):
+            z = q_of_z.rsample([chunk])
+            zs.append(z)
+            log_p_z.append(self.prior_log_prob(z).reshape(chunk, -1))
+            log_q_z.append(q_of_z.log_prob(z).sum(dim=-1).reshape(chunk, -1))
+        log_p_x = self.log_p_x_given_z(x, torch.cat(zs), labels[..., 1:], padding, samples_per_pass)
+        return (torch.cat(log_p_z) + log_p_x - torch.cat(log_q_z)).logsumexp(dim=0) - math.log(num_samples)
+
+    def log_p_x_given_z(self, x: Tensor, z: Tensor, labels: Tensor, padding: Optional[Tensor] = None,
+                        samples_per_pass: Optional[int] = None) -> Tensor:
+        """log p(x | z_s) for latent samples z [S, B, 1, latent]: [S, B] fp32, the fast path of estimate_log_prob_iw
+        (one decoder pass per group of samples stacked sample-major along the batch, `fused_ce.vocab_log_prob`)."""
+        x, x_pad = split_padding(x)
+        padding = x_pad if padding is None else padding
+        S, B, L = z.shape[0], x.shape[0], x.shape[1]
+        group = samples_per_pass or max(1, self.IW_TOKENS_PER_PASS // (B * L))
+        out = []
+        for s0 in range(0, S, group):
+            g = min(group, S - s0)
+            xg = x.repeat(g, 1, 1) if g > 1 else x
+            pg = padding.repeat(g, 1) if (padding is not None and g > 1) else padding
+            zg = z[s0:s0 + g].reshape(g * B, *z.shape[2:])
+            hidden = self.reconstruct(xg, zg, padding=pg, return_hidden=True)
+            lp = fused_ce.vocab_log_prob(hidden, self.output_layer[-1], labels.repeat(g, 1) if g > 1 else labels)
+            out.append(lp.sum(dim=-1).reshape(g, B))
+        return torch.cat(out)
 
     def predict(self, batch: Any, batch_idx: int = 0, dataloader_idx: Optional[int] = None):
         tokens, padding = split_padding(batch['token_ids'])
