@@ -9,6 +9,7 @@ run t1_bottleneck python -m pytest tests/test_gpu_bottleneck.py -q --no-header -
 run t2_exact python -m pytest tests/test_gpu_attention.py -q --no-header -rfE -p no:cacheprovider -k "exact"
 run t3_dump python -m pytest tests/test_gpu_attention.py -q --no-header -rfE -p no:cacheprovider -k "raw_scores"
 run t4_sm100 python -m pytest tests/test_gpu_attention.py -q --no-header -rfE -p no:cacheprovider -k "sm100 and not raw_scores or masked or validation"
+run t4b_probes python -m pytest tests/test_gpu_attention_probes.py -q --no-header -rfE -p no:cacheprovider
 run t5_full python -m pytest tests/test_gpu_attention.py -q --no-header -rfE -p no:cacheprovider -k "full_size"
 run t6_model python -m pytest tests/test_gpu_model.py -q --no-header -rfE -p no:cacheprovider
 run t7_smoke python -c "import __graft_entry__ as g; g.smoke()"
