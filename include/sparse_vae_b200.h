@@ -339,6 +339,25 @@ SVAE_API int svae_decode_attn(const void* q, const void* k, const void* v, const
                      const int32_t* position, int32_t B, int32_t H, int32_t head_dim, int32_t window, int32_t block,
                      int32_t table_rows, int64_t in_stride, int32_t dtype, float scale, void* stream);
 
+/* The same step for a DENSE causal attention layer (reference core/attention.py:107-142 with `cfg is None`): rotary
+ * of the new q / k rows at the DEVICE counter `position` (same arithmetic and tables as svae_decode_attn), append of
+ * k / v at slot `position`, and attention of the new query over slots 0..position (fp32 softmax and accumulation).
+ *   q, k, v, out, cos_table, sin_table  as for svae_decode_attn
+ *   key_cache, value_cache [B, cache_len, H*head_dim] `dtype`: slot p holds position p (the reference's cache), so the
+ *                         first tokens may be decoded by the ATen path.
+ *   workspace             svae_decode_attn_dense_workspace_bytes(B, H, head_dim, cache_len) bytes, 16-byte aligned
+ *                         (may be null when that is 0); holds the per-split partial results.
+ * Split-KV: the live slots are dealt out to a number of CTAs per (sample, head) fixed by B, H and cache_len, and their
+ * partial softmax results are merged in a fixed order (no atomics): bit-identical from run to run, graph-capturable.
+ * position >= cache_len reads and writes nothing.  head_dim 32 | 64, cache_len 1..65536. */
+SVAE_API int svae_decode_attn_dense_supported(int32_t head_dim, int32_t cache_len);
+SVAE_API size_t svae_decode_attn_dense_workspace_bytes(int32_t B, int32_t H, int32_t head_dim, int32_t cache_len);
+SVAE_API int svae_decode_attn_dense(const void* q, const void* k, const void* v, const float* cos_table,
+                           const float* sin_table, void* key_cache, void* value_cache, void* out,
+                           const int32_t* position, void* workspace, size_t workspace_bytes, int32_t B, int32_t H,
+                           int32_t head_dim, int32_t cache_len, int32_t table_rows, int64_t in_stride, int32_t dtype,
+                           float scale, void* stream);
+
 /* Residual-stream update under autocast (reference core/transformer_layer.py:41,49,61 `x = x + h`): out = x + h with
  * x, out fp32 and h 16-bit, numel % 8 == 0, 16-byte aligned; out == x is allowed. */
 SVAE_API int svae_residual_add(const float* x, const void* h, int32_t h_dtype, float* out, int64_t numel, void* stream);

@@ -40,7 +40,8 @@ EXPORTS = (
     'svae_multi_tensor_chunks', 'svae_multi_tensor_scale_copy', 'svae_clip_grad_norm', 'svae_radam_step',
     'svae_vocab_ce_supported', 'svae_vocab_ce', 'svae_rotary', 'svae_colsum_workspace_floats', 'svae_colsum_counters', 'svae_colsum',
     'svae_layernorm_supported', 'svae_layernorm_fwd', 'svae_layernorm_bwd_workspace_floats', 'svae_layernorm_bwd',
-    'svae_decode_attn_supported', 'svae_decode_attn', 'svae_sample_top_p_supported', 'svae_sample_top_p',
+    'svae_decode_attn_supported', 'svae_decode_attn', 'svae_decode_attn_dense_supported',
+    'svae_decode_attn_dense_workspace_bytes', 'svae_decode_attn_dense', 'svae_sample_top_p_supported', 'svae_sample_top_p',
     'svae_residual_layernorm', 'svae_residual_add', 'svae_multi_tensor_cast', 'svae_residual_dropout_add',
     'svae_dropout_branch_grad', 'svae_bottleneck_fwd_g', 'svae_bottleneck_bwd_g', 'svae_residual_dropout_add_g',
     'svae_dropout_branch_grad_g', 'svae_radam_args_bytes', 'svae_radam_args', 'svae_radam_step_g',
@@ -161,6 +162,13 @@ def _load() -> C.CDLL:
     lib.svae_decode_attn_supported.argtypes = [i32, i32, i32]
     lib.svae_decode_attn.restype = C.c_int
     lib.svae_decode_attn.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i64, i32, C.c_float, vp]
+    lib.svae_decode_attn_dense_supported.restype = C.c_int
+    lib.svae_decode_attn_dense_supported.argtypes = [i32, i32]
+    lib.svae_decode_attn_dense_workspace_bytes.restype = C.c_size_t
+    lib.svae_decode_attn_dense_workspace_bytes.argtypes = [i32, i32, i32, i32]
+    lib.svae_decode_attn_dense.restype = C.c_int
+    lib.svae_decode_attn_dense.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, i32, i32, i32, i32, i32, i64,
+                                           i32, C.c_float, vp]
     lib.svae_residual_dropout_add.restype = C.c_int
     lib.svae_residual_dropout_add.argtypes = [vp, vp, i32, vp, i64, C.c_float, C.c_uint64, C.c_uint64, vp]
     lib.svae_dropout_branch_grad.restype = C.c_int

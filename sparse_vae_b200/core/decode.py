@@ -1,4 +1,5 @@
-"""CUDA-graphed token-by-token decoding for `TransformerVAE.sample` (SURVEY.md section 8f row 3).
+"""CUDA-graphed token-by-token decoding for `TransformerVAE.sample` and `TransformerLanguageModel.sample` (SURVEY.md
+section 8f row 3).
 
 The reference's sampler (transformer_vae.py:112-126 driving core/attention.py:107-168 and core/generation.py:30-77)
 issues ~400 small launches per token and synchronises with the host several times per token (boolean-mask indexing,
@@ -9,15 +10,19 @@ whole decoder is ONE graph replay:
     output column) is read from device counters that the graph itself advances;
   * each sparse-attention layer is one launch of `svae_decode_attn` (csrc/decode_attn.cu): rotary + cache append +
     attention over the visible keys; q / k / v come from one fused [3D, D] projection;
+  * each dense causal layer (`sparse_self_attention=False`) is one call of `svae_decode_attn_dense`
+    (csrc/decode_attn_dense.cu): the same over the reference's growing [B, max_length, D] cache, split-KV;
   * `GenerationState.process_logits` is restated with fixed shapes (same ops, same order, same RNG consumption).
 
   * with the reference's default settings (nucleus sampling) the sampler itself is one launch (csrc/sampling.cu):
     threshold search instead of a full sort; same token distribution, its own use of the random stream.
 
 Finished samples leave the batch like in the reference (their cache rows are dropped and the rest is compacted,
-`Attention.update_kv_cache`) -- but not after every token: they first stay behind as dead rows (nothing written, not
-counted again) and the batch is compacted and the graph re-captured once a quarter of it is dead (`COMPACT_BELOW`).
-The first token (position 0, where every layer's input is its own projection of z) runs through the unfused modules.
+`Attention.update_kv_cache`; a dense layer's cache only over the slots written so far) -- but not after every token:
+they first stay behind as dead rows (nothing written, not counted again) and the batch is compacted and the graph
+re-captured once a quarter of it is dead (`COMPACT_BELOW`).
+The first token (position 0, where every layer's input is its own projection of z) runs through the unfused modules,
+which also allocates the caches.
 Weights are frozen while sampling: they are cast to the autocast dtype once per call instead of once per token.
 """
 from __future__ import annotations
@@ -41,23 +46,31 @@ COMPACT_BELOW = 0.75
 CHECK_EVERY = 8
 
 
+def attention_kind(layer, cache_len: int) -> Optional[str]:
+    """How one decoder layer's self-attention is decoded by the graphed sampler: 'sparse' (`svae_decode_attn` over the
+    ring cache), 'dense' (`svae_decode_attn_dense` over the reference's [B, cache_len, D] cache) or None (not covered:
+    cross-attention, learned queries, non-causal attention or an unsupported head size / length)."""
+    attn = layer.attention
+    if layer.cross_attention is not None or attn.learned_queries is not None:
+        return None
+    head_dim = attn.d_model // attn.num_heads
+    cfg = attn.sparse_attention
+    if cfg is None:
+        return 'dense' if attn.causal and N.lib.svae_decode_attn_dense_supported(head_dim, cache_len) else None
+    if cfg.causal and cfg.include_cls and N.lib.svae_decode_attn_supported(head_dim, int(cfg.window_size), cfg.block_size):
+        return 'sparse'
+    return None
+
+
 def supported(model, state: GenerationState) -> bool:
-    """Graphed decoding covers the default model family: CUDA, every decoder layer block-sparse (causal, global first
-    block) without cross-attention, head size 32 or 64.  Anything else keeps the module-by-module sampler."""
+    """Graphed decoding covers CUDA models whose every decoder layer is causal self-attention without cross-attention,
+    either block-sparse (global first block) or dense, head size 32 or 64.  Anything else keeps the module-by-module
+    sampler."""
     if not (N.FUSED_EXTRAS and model.device.type == 'cuda' and len(model.decoder_layers) > 0):
         return False
     if len(model.input_layer) != 2 or state.output_ids.dtype != torch.long:
         return False
-    for layer in model.decoder_layers:
-        attn = layer.attention
-        cfg = attn.sparse_attention
-        if cfg is None or layer.cross_attention is not None or attn.learned_queries is not None:
-            return False
-        if not (cfg.causal and cfg.include_cls):
-            return False
-        if not N.lib.svae_decode_attn_supported(attn.d_model // attn.num_heads, int(cfg.window_size), cfg.block_size):
-            return False
-    return True
+    return all(attention_kind(layer, state.output_ids.shape[1]) is not None for layer in model.decoder_layers)
 
 
 class _LayerWeights:
@@ -80,14 +93,21 @@ class GraphedDecoder:
         dev = model.device
         self.dtype = torch.get_autocast_dtype('cuda') if torch.is_autocast_enabled('cuda') else torch.float32
         self.max_length = state.output_ids.shape[1]
-        attn = model.decoder_layers[0].attention
-        cfg = attn.sparse_attention
-        self.heads, self.head_dim = attn.num_heads, attn.d_model // attn.num_heads
-        self.window, self.block = int(cfg.window_size), cfg.block_size
-        max_pos = 2 * self.window * self.block
-        # row p = the one-row table the reference builds at offset p (positions rounded to the activation dtype)
-        cos, sin = _rotary_tables(self.max_length, attn.d_model // 2, 0, max_pos, self.dtype, dev)
-        self.cos, self.sin = cos.float().contiguous(), sin.float().contiguous()
+        # per layer: 'sparse' or 'dense' (tests read this), and the rotary tables of its max_pos -- 2*window*block for
+        # sparse layers, attn.max_length for dense ones; row p = the one-row table the reference builds at offset p
+        # (positions rounded to the activation dtype)
+        self.attention_kinds = [attention_kind(layer, self.max_length) for layer in model.decoder_layers]
+        tables = {}
+        self.tables = []
+        for layer, kind in zip(model.decoder_layers, self.attention_kinds):
+            attn = layer.attention
+            cfg = attn.sparse_attention
+            max_pos = 2 * int(cfg.window_size) * cfg.block_size if kind == 'sparse' else attn.max_length
+            if max_pos not in tables:
+                cos, sin = _rotary_tables(self.max_length, attn.d_model // 2, 0, max_pos, self.dtype, dev)
+                tables[max_pos] = (cos.float().contiguous(), sin.float().contiguous())
+            self.tables.append(tables[max_pos])
+        self.workspace = None       # split-KV partials of the dense layers, sized for the captured batch
         self.layers = [_LayerWeights(layer, self.dtype) for layer in model.decoder_layers]
         head = model.output_layer
         self.head_w0, self.head_b0 = head[0].weight.to(self.dtype), head[0].bias.to(self.dtype)
@@ -112,17 +132,29 @@ class GraphedDecoder:
         self.captures = 0
 
     # ---- one token, fixed shapes (this is what gets captured) ------------------------------------------------
-    def _attend(self, module: Attention, w: _LayerWeights, h: Tensor) -> Tensor:
+    def _attend(self, i: int, module: Attention, w: _LayerWeights, h: Tensor) -> Tensor:
         B, D = h.shape[0], module.d_model
+        heads = module.num_heads
+        head_dim = D // heads
         qkv = F.linear(h, w.wqkv, w.bqkv)                                   # [B, 1, 3D]
         out = torch.empty(B, 1, D, dtype=qkv.dtype, device=qkv.device)
         flat = qkv.view(B, 3 * D)
-        N.check(N.lib.svae_decode_attn(flat[:, :D].data_ptr(), flat[:, D:2 * D].data_ptr(), flat[:, 2 * D:].data_ptr(),
-                                       self.cos.data_ptr(), self.sin.data_ptr(), module.key_cache.data_ptr(),
-                                       module.value_cache.data_ptr(), out.data_ptr(), self.position.data_ptr(), B,
-                                       self.heads, self.head_dim, self.window, self.block, self.max_length, 3 * D,
-                                       N.svae_dtype(qkv.dtype), float(self.head_dim ** -0.5),
-                                       N.current_stream(qkv.device)), 'svae_decode_attn')
+        cos, sin = self.tables[i]
+        stream = N.current_stream(qkv.device)
+        if self.attention_kinds[i] == 'dense':
+            N.check(N.lib.svae_decode_attn_dense(
+                flat[:, :D].data_ptr(), flat[:, D:2 * D].data_ptr(), flat[:, 2 * D:].data_ptr(), cos.data_ptr(),
+                sin.data_ptr(), module.key_cache.data_ptr(), module.value_cache.data_ptr(), out.data_ptr(),
+                self.position.data_ptr(), N.ptr(self.workspace), self.workspace.numel(), B, heads, head_dim,
+                module.key_cache.shape[1], cos.shape[0], 3 * D, N.svae_dtype(qkv.dtype), float(head_dim ** -0.5),
+                stream), 'svae_decode_attn_dense')
+        else:
+            cfg = module.sparse_attention
+            N.check(N.lib.svae_decode_attn(flat[:, :D].data_ptr(), flat[:, D:2 * D].data_ptr(), flat[:, 2 * D:].data_ptr(),
+                                           cos.data_ptr(), sin.data_ptr(), module.key_cache.data_ptr(),
+                                           module.value_cache.data_ptr(), out.data_ptr(), self.position.data_ptr(), B,
+                                           heads, head_dim, int(cfg.window_size), cfg.block_size, self.max_length, 3 * D,
+                                           N.svae_dtype(qkv.dtype), float(head_dim ** -0.5), stream), 'svae_decode_attn')
         return F.linear(out, w.wo, w.bo)
 
     def _add_norm(self, x: Tensor, h: Tensor, norm) -> Tensor:
@@ -179,7 +211,7 @@ class GraphedDecoder:
         y = model.decoder_layers[0].attn_layer_norm(x)
         last = len(self.layers) - 1
         for i, (layer, w) in enumerate(zip(model.decoder_layers, self.layers)):
-            y = self._add_norm(x, self._attend(layer.attention, w, y), layer.ffn_layer_norm)
+            y = self._add_norm(x, self._attend(i, layer.attention, w, y), layer.ffn_layer_norm)
             h = layer.dropout(F.linear(F.gelu(F.linear(y, w.w1, w.b1)), w.w2))
             if i < last:
                 y = self._add_norm(x, h, model.decoder_layers[i + 1].attn_layer_norm)
@@ -218,6 +250,11 @@ class GraphedDecoder:
         self.alive = torch.ones(self.rows.numel(), dtype=torch.bool, device=self.ids.device)
         self.position.fill_(st.current_index - 1)
         self.column.fill_(st.current_index)
+        B = self.rows.numel()
+        self.workspace = torch.empty(max([N.lib.svae_decode_attn_dense_workspace_bytes(
+            B, layer.attention.num_heads, layer.attention.d_model // layer.attention.num_heads, self.max_length)
+            for layer, kind in zip(self.model.decoder_layers, self.attention_kinds) if kind == 'dense'] + [0]),
+            dtype=torch.uint8, device=self.ids.device)
         if self.trace is not None:
             self.trace_buffer = torch.empty(self.rows.numel(), self.head_w3.shape[0], dtype=self.dtype,
                                             device=self.ids.device)
@@ -234,8 +271,25 @@ class GraphedDecoder:
         st.output_ids[self.rows] = self.ids
         if drop_finished:
             st.live_sample_mask[self.rows] = self.alive
-            Attention.update_kv_cache(self.alive)
+            self._compact_caches(self.alive)
         self.graph = None
+
+    def _compact_caches(self, keep: Tensor):
+        """Attention.update_kv_cache for the graphed decoder: sparse layers' ring caches are gathered as there; a dense
+        layer's [B, max_length, D] cache is compacted in place over the slots written so far (0..current_index-2),
+        not over all max_length of them -- the slots beyond are still zero in every row."""
+        if 'dense' not in self.attention_kinds:
+            Attention.update_kv_cache(keep)
+            return
+        live, end = int(keep.sum()), self.state.current_index - 1
+        for module in Attention.live_attention_modules:
+            if module.sparse_attention is None:
+                for cache in (module.key_cache, module.value_cache):
+                    cache[:live, :end] = cache[keep, :end]
+                module.key_cache, module.value_cache = module.key_cache[:live], module.value_cache[:live]
+            else:
+                module.key_cache = module.key_cache[keep, ...]
+                module.value_cache = module.value_cache[keep, ...]
 
     @torch.no_grad()
     def run(self):

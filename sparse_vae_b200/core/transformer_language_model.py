@@ -10,6 +10,7 @@ from typing import Dict, Optional
 import torch
 from torch import nn, Tensor
 
+from . import decode
 from .attention import Attention, TransformerLayer
 from .embedding import Embedding
 from .gelu import GELU
@@ -84,6 +85,9 @@ class TransformerLanguageModel(LanguageModel):
         context = self.embed_context(context) if context is not None else None
         state = GenerationState(max_length, batch_size, self.start_token, self.end_token, device=self.device, **kwargs)
         state.output_ids[:, 0] = self.start_token
+        # after the first token (which allocates the caches) every token is one graph replay (core/decode.py), as in
+        # TransformerVAE.sample; z or context added to the input keep the module-by-module sampler
+        graphed = z is None and context is None and decode.supported(self, state)
         with Attention.kv_cache(max_length):
             while not state.should_stop():
                 x = self.input_layer(state.prev_tokens())
@@ -92,4 +96,7 @@ class TransformerLanguageModel(LanguageModel):
                 for layer in self.decoder_layers:
                     x = layer(x, context=context)
                 Attention.update_kv_cache(state.process_logits(self.output_layer(x.squeeze(1))))
+                if graphed:
+                    decode.GraphedDecoder(self, state, decode.TRACE).run()
+                    break
         return state.final_output()
