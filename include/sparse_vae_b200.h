@@ -119,8 +119,8 @@ SVAE_API int svae_attn_bwd(const svae_attn_desc* desc, const void* q, const void
 
 /* Test hook (no global state): variant of svae_attn_fwd for the tcgen05 path.  s_dump (may be NULL): raw scores S = q k^T (before
  * scale/masks) of every query row against its tile's key slots, [batch, heads, seq_len, slots*32] fp32
- * (slots = svae_attn_fwd_slots(desc)).  timeline (may be NULL): int64 [num_ctas, 5, 8] per-warp clock64
- * stamps of the kernel's phases (CTA order: batch, head, tile). */
+ * (slots = svae_attn_fwd_slots(desc)).  timeline must be NULL: the argument is kept for ABI compatibility, and a
+ * non-NULL timeline returns SVAE_ERR_UNSUPPORTED. */
 SVAE_API int svae_attn_fwd_slots(const svae_attn_desc* desc);
 SVAE_API int svae_attn_fwd_debug(const svae_attn_desc* desc, const void* q, const void* k, const void* v,
                         const float* key_padding_mask, void* out, float* lse, float* s_dump,

@@ -12,10 +12,7 @@ from pathlib import Path
 import torch
 
 _HERE = Path(__file__).resolve().parent
-import os as _os
-
-# SVAE_LIB_VARIANT=<suffix>: an experimental build of the same library (csrc/build.py --variant), kernel experiments only
-LIB_PATH = _HERE / 'csrc' / f"libsvae_b200{_os.environ.get('SVAE_LIB_VARIANT', '')}.so"
+LIB_PATH = _HERE / 'csrc' / 'libsvae_b200.so'
 
 DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
 ATTN_FORCE_EXACT = 1
@@ -201,19 +198,6 @@ def _load() -> C.CDLL:
 
 
 lib = _load()
-
-
-def load_debug() -> C.CDLL:
-    """libsvae_b200_dbg.so (include/sparse_vae_b200_debug.h): micro-benchmarks, never loaded by the product path."""
-    path = _HERE / 'csrc' / 'libsvae_b200_dbg.so'
-    if not path.exists():
-        raise ImportError(f"{path} is missing: build it with `python sparse_vae_b200/csrc/build.py --debug`")
-    dbg = C.CDLL(str(path))
-    for name in ('svae_debug_mma_bench', 'svae_debug_pipe_bench'):
-        fn = getattr(dbg, name)
-        fn.restype = C.c_int
-        fn.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
-    return dbg
 
 
 def check(rc: int, what: str):

@@ -47,29 +47,6 @@ using namespace ptx;
 constexpr int kB1Threads = 512;
 constexpr int kB1MaxLeft = 4;
 
-// Debug builds (libsvae_b200_dbg.so, -DSVAE_DEBUG_BUILD) account the cycles every warp spends in each kind of wait;
-// the product build compiles the plain wait.
-#ifdef SVAE_DEBUG_BUILD
-int g_b1_knock = 0;      // knock-out experiments (results are wrong): 1 math as if every unit were dead, 2 no dQ / global MMAs,
-                         // 4 no accumulator drain / stores, 8 no dV / dK MMAs, 16 S^T / dP^T with one k-step, 32 no statistics
-#define B1_KNOCK(bit) (p.knock & (bit))
-long long* g_b1_timeline = nullptr;      // [num_ctas][16 warps][16]: waits by kind, [10] = total, [11] = tiles, [12..15] = role-specific spans
-#define B1_WAIT(kind, bar, parity)                    \
-  do {                                                \
-    if (tl_on) {                                      \
-      const long long _t0 = clock64();                \
-      mbar_wait(bar, parity);                    \
-      tl_acc[kind] += clock64() - _t0;                \
-    } else {                                          \
-      mbar_wait(bar, parity);                    \
-    }                                                 \
-  } while (0)
-#else
-#define B1_WAIT(kind, bar, parity) mbar_wait(bar, parity)
-#define B1_KNOCK(bit) false
-#endif
-enum : int { W_FULL = 0, W_STAT = 1, W_SREADY = 2, W_PREADY = 3, W_UFREE = 4, W_GRP = 5, W_DSFREE = 6, W_ACCREADY = 7, W_ACCFREE = 8, W_FREE = 9 };
-
 template <int DH>
 struct B1Smem {
   static constexpr int ROWB = DH * 2;
@@ -102,8 +79,6 @@ struct B1Params {
   int left, cls, nq;       // band width, global column, slots per key tile (left + 3)
   int num_tiles, num_ctas;
   float scale, scale_log2;
-  long long* timeline;     // debug builds only
-  int knock;               // debug builds only
 };
 
 // first tile of CTA i's range
@@ -219,11 +194,6 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
 
   const int warp = warp_index(), lane = threadIdx.x & 31;
   const B1Geom g(p);
-#ifdef SVAE_DEBUG_BUILD
-  long long tl_acc[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  const long long tl_start = clock64();
-  const bool tl_on = p.timeline != nullptr;
-#endif
 
   auto init_barriers = [&]() {
     auto init_n = [&](int first, int n, uint32_t count) { for (int i = 0; i < n; ++i) mbar_init(bars + first + i, count); };
@@ -287,30 +257,18 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           bool pre;
           g.tile(s, j, kt, pre, ub, ue);
           const int sl = j & 1;
-          if (j >= 2) B1_WAIT(W_FREE, bars + BAR_V_FREE + sl, ((j - 2) >> 1) & 1);
-          if (B1_KNOCK(64)) {
-            mbar_arrive_expect_tx_w(bars + BAR_V_FULL + sl, 0);
-          } else {
-            mbar_arrive_expect_tx_w(bars + BAR_V_FULL + sl, S::TILE);
-            tma_load_4d_w(smem + S::OFF_V + sl * S::TILE, &tmV, bars + BAR_V_FULL + sl, 0, kt * kTile, s.h, s.b);
-          }
-          if (j >= 2) B1_WAIT(W_FREE, bars + BAR_K_FREE + sl, ((j - 2) >> 1) & 1);
-          if (B1_KNOCK(64)) {
-            mbar_arrive_expect_tx_w(bars + BAR_K_FULL + sl, 0);
-          } else {
-            mbar_arrive_expect_tx_w(bars + BAR_K_FULL + sl, S::TILE);
-            tma_load_4d_w(smem + S::OFF_K + sl * S::TILE, &tmK, bars + BAR_K_FULL + sl, 0, kt * kTile, s.h, s.b);
-          }
+          if (j >= 2) mbar_wait(bars + BAR_V_FREE + sl, ((j - 2) >> 1) & 1);
+          mbar_arrive_expect_tx_w(bars + BAR_V_FULL + sl, S::TILE);
+          tma_load_4d_w(smem + S::OFF_V + sl * S::TILE, &tmV, bars + BAR_V_FULL + sl, 0, kt * kTile, s.h, s.b);
+          if (j >= 2) mbar_wait(bars + BAR_K_FREE + sl, ((j - 2) >> 1) & 1);
+          mbar_arrive_expect_tx_w(bars + BAR_K_FULL + sl, S::TILE);
+          tma_load_4d_w(smem + S::OFF_K + sl * S::TILE, &tmK, bars + BAR_K_FULL + sl, 0, kt * kTile, s.h, s.b);
           // query tiles this key tile touches: kt (local kt - t0; not for the pre-tile) and kt + 1 (slots 4..)
           int need = g.has_y(ue) ? (kt + 1 - s.t0) + 1 : (kt - s.t0) + 1;
           if (need > s.nqt) need = s.nqt;
           for (; qnext < need; ++qnext) {
             const int n = qnext, r = n % 3;
-            if (n >= 3) B1_WAIT(W_FREE, bars + BAR_RING_FREE + r, ((n - 3) / 3) & 1);
-            if (B1_KNOCK(64)) {
-              mbar_arrive_expect_tx_w(bars + BAR_Q_FULL + r, 0);
-              continue;
-            }
+            if (n >= 3) mbar_wait(bars + BAR_RING_FREE + r, ((n - 3) / 3) & 1);
             mbar_arrive_expect_tx_w(bars + BAR_Q_FULL + r, 2 * S::TILE);
             tma_load_4d_w(ring_do(n), &tmDO, bars + BAR_Q_FULL + r, 0, (s.t0 + n) * kTile, s.h, s.b);
             tma_load_4d_w(ring_q(n), &tmQ, bars + BAR_Q_FULL + r, 0, (s.t0 + n) * kTile, s.h, s.b);
@@ -333,15 +291,15 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           g.tile(s, j, kt, pre, ub, ue);
           const int sl = j & 1;
           const uint32_t k_addr = smem_u32(smem + S::OFF_K + sl * S::TILE), v_addr = smem_u32(smem + S::OFF_V + sl * S::TILE);
-          B1_WAIT(W_FULL, bars + BAR_K_FULL + sl, (j >> 1) & 1);
-          B1_WAIT(W_FULL, bars + BAR_V_FULL + sl, (j >> 1) & 1);
+          mbar_wait(bars + BAR_K_FULL + sl, (j >> 1) & 1);
+          mbar_wait(bars + BAR_V_FULL + sl, (j >> 1) & 1);
           for (int pos = ub; pos < ue; ++pos, ++u) {
             const int buf = u & 1;                                           // = the math group that owns the unit
             const int slot = g.slot_of(pos);
             const int n = (kt - s.t0) + (slot < 0 ? 0 : (slot >> 2));       // local query tile of the unit
-            for (; q_waited <= n; ++q_waited) B1_WAIT(W_FULL, bars + BAR_Q_FULL + q_waited % 3, (q_waited / 3) & 1);
-            if (slot < 0 && !k0_waited) { B1_WAIT(W_FULL, bars + BAR_K0_FULL, 0); k0_waited = true; }
-            if (u >= 2) B1_WAIT(W_UFREE, bars + BAR_U_FREE + buf, ((u - 2) >> 1) & 1);
+            for (; q_waited <= n; ++q_waited) mbar_wait(bars + BAR_Q_FULL + q_waited % 3, (q_waited / 3) & 1);
+            if (slot < 0 && !k0_waited) { mbar_wait(bars + BAR_K0_FULL, 0); k0_waited = true; }
+            if (u >= 2) mbar_wait(bars + BAR_U_FREE + buf, ((u - 2) >> 1) & 1);
             tc_fence_after();
             const uint32_t d_s = tmem_base + S::COL_U + 64 * buf, d_dp = d_s + 32;
             const uint32_t q_addr = smem_u32(ring_q(n)), do_addr = smem_u32(ring_do(n));
@@ -353,7 +311,6 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             }
 #pragma unroll
             for (int ks = 0; ks < DH / 16; ++ks) {
-              if ((ks > 0 && B1_KNOCK(16)) || B1_KNOCK(256)) break;
               mma_ss_w(d_s, make_smem_desc(a_s + ks * 32, 16, 8 * ROWB, ROWB), make_smem_desc(b_s + ks * 32, 16, 8 * ROWB, ROWB),
                        idesc_s, ks > 0 ? 1u : 0u);
               mma_ss_w(d_dp, make_smem_desc(a_dp + ks * 32, 16, 8 * ROWB, ROWB), make_smem_desc(b_dp + ks * 32, 16, 8 * ROWB, ROWB),
@@ -380,12 +337,12 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           for (int pos = ub; pos < ue; ++pos, ++u) {
             const int buf = u & 1;
             const int slot = g.slot_of(pos);
-            B1_WAIT(W_PREADY, bars + BAR_P_READY + buf, (u >> 1) & 1);      // every phase is observed, in order
+            mbar_wait(bars + BAR_P_READY + buf, (u >> 1) & 1);      // every phase is observed, in order
             if (slot < 0) continue;                     // the global unit's MMAs belong to warp 15
-            if (!pre && !B1_KNOCK(8)) {
+            if (!pre) {
               // (the epilogue arrives once per tile, pre-tiles included: it has then seen the previous tile's
               //  ACC_READY / ACC_READY2 phases, so those barriers can never run two phases ahead of their waiter)
-              if (acc == 0 && j >= 1) B1_WAIT(W_ACCFREE, bars + BAR_ACC_FREE, (j - 1) & 1);
+              if (acc == 0 && j >= 1) mbar_wait(bars + BAR_ACC_FREE, (j - 1) & 1);
               tc_fence_after();
               const int n = (kt - s.t0) + (slot >> 2);
               const uint32_t q_addr = smem_u32(ring_q(n)) + (slot & 3) * S::SLOT, do_addr = smem_u32(ring_do(n)) + (slot & 3) * S::SLOT;
@@ -424,12 +381,12 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           const uint32_t acc_x = tmem_base + S::COL_DQ + 64 * (kt & 1), acc_y = tmem_base + S::COL_DQ + 64 * ((kt + 1) & 1);
           // dQ (+)= dS K over the 128 keys of the tile: A = staged dS^T read MN-major (two 64-query halves 16 KB apart)
           auto issue_dq = [&](uint32_t d, uint32_t first_acc, uint64_t* ready, int& count) {
-            B1_WAIT(W_GRP, ready, count & 1);
+            mbar_wait(ready, count & 1);
             ++count;
             tc_fence_after();
 #pragma unroll
             for (int k2 = 0; k2 < kTile / 16; ++k2)
-              if (!B1_KNOCK(2)) mma_ss_w(d, make_smem_desc(ds_addr + k2 * 16 * 128, S::TILE, 8 * 128, 128),
+              mma_ss_w(d, make_smem_desc(ds_addr + k2 * 16 * 128, S::TILE, 8 * 128, 128),
                        make_smem_desc(k_addr + k2 * 16 * ROWB, S::SLOT, 8 * ROWB, ROWB), idesc_mn, k2 > 0 ? 1u : first_acc);
             tc_commit_w(bars + BAR_DS_FREE);
           };
@@ -439,19 +396,19 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             if (slot == g.nx - 1) issue_dq(acc_x, prev_y ? 1u : 0u, bars + BAR_GRPX_READY, xgroups);
             if (slot >= 4 && slot == g.nq - 1) issue_dq(acc_y, 0u, bars + BAR_GRPY_READY, ygroups);
             if (slot < 0) {
-              B1_WAIT(W_PREADY, bars + BAR_P_READY + buf, (u >> 1) & 1);
+              mbar_wait(bars + BAR_P_READY + buf, (u >> 1) & 1);
               tc_fence_after();
               const int n = kt - s.t0;
               const uint32_t do_addr = smem_u32(ring_do(n));
               const uint32_t ta = tmem_base + S::COL_A + 32 * buf;
 #pragma unroll
               for (int k2 = 0; k2 < 2; ++k2)            // dQ X += dS_g K_0
-                if (!B1_KNOCK(2)) mma_ts_w(acc_x, ta + 8 * k2, make_smem_desc(k0_addr + k2 * 16 * ROWB, S::SLOT, 8 * ROWB, ROWB), idesc_o, 1u);
+                mma_ts_w(acc_x, ta + 8 * k2, make_smem_desc(k0_addr + k2 * 16 * ROWB, S::SLOT, 8 * ROWB, ROWB), idesc_o, 1u);
               // G (+)= [dO^T ; Q^T] (128 x 128 queries) [P_g | dS_g] (128 queries x 64): rows 0-63 x columns 0-31 = dV_0^T,
               // rows 64-127 x columns 32-63 = dK_0^T
 #pragma unroll
               for (int k2 = 0; k2 < kTile / 16; ++k2)
-                if (!B1_KNOCK(2)) mma_ss_w(tmem_base + S::COL_G, make_smem_desc(do_addr + k2 * 16 * ROWB, S::TILE, 8 * ROWB, ROWB),
+                mma_ss_w(tmem_base + S::COL_G, make_smem_desc(do_addr + k2 * 16 * ROWB, S::TILE, 8 * ROWB, ROWB),
                          make_smem_desc(g_addr + k2 * 16 * 128, 16 * 128, 8 * 128, 128), idesc_mn, (k2 > 0 || gtiles > 0) ? 1u : 0u);
               tc_commit_w(bars + BAR_A_FREE + buf);
               tc_commit_w(bars + BAR_G_FREE);
@@ -496,7 +453,7 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           const int qpos = q0 + ps * 16 + rsub;
           ov[ps] = make_uint4(0, 0, 0, 0);
           lv[ps] = 0.f;
-          if (qpos < p.L && !B1_KNOCK(32)) {
+          if (qpos < p.L) {
             ov[ps] = __ldg(reinterpret_cast<const uint4*>(o_seq + (int64_t)qpos * p.o_stride[2]) + chunk);
             if (chunk == 0) lv[ps] = __ldg(p.lse + stat_base + qpos);
           }
@@ -504,7 +461,7 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       };
       auto stats_finish = [&](int n) {
         const int r = n % 3;
-        B1_WAIT(W_FULL, bars + BAR_Q_FULL + r, (n / 3) & 1);
+        mbar_wait(bars + BAR_Q_FULL + r, (n / 3) & 1);
         const uint8_t* sdo = ring_do(n);
         float* st = sStat + r * 2 * kTile;
 #pragma unroll
@@ -549,17 +506,10 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
         const int pending = stats_done < want ? stats_done : -1;
         if (pending >= 0) stats_issue(pending);
 
-        B1_WAIT(W_ACCREADY, bars + BAR_ACC_READY, j & 1);
-        B1_WAIT(W_ACCREADY, bars + BAR_ACC_READY2, j & 1);
+        mbar_wait(bars + BAR_ACC_READY, j & 1);
+        mbar_wait(bars + BAR_ACC_READY2, j & 1);
         tc_fence_after();
-        if (!pre && B1_KNOCK(4)) {
-          tc_fence_before();
-          mbar_arrive_warp(bars + BAR_ACC_FREE);
-          if (tid_g == 0) {
-            mbar_arrive(bars + BAR_K_FREE + (j & 1));
-            mbar_arrive(bars + BAR_RING_FREE + (kt - s.t0) % 3);
-          }
-        } else if (!pre) {
+        if (!pre) {
           const int n = kt - s.t0;
           uint8_t* stage[3] = {smem + S::OFF_K + (j & 1) * S::TILE, ring_do(n), ring_q(n)};        // dK, dV, dQ
           const uint32_t cols[3] = {(uint32_t)S::COL_DK, (uint32_t)S::COL_DV, (uint32_t)(S::COL_DQ + 64 * (kt & 1))};
@@ -656,7 +606,7 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           if (slot < 0) ++gtiles;
           if ((u & 1) != wg) continue;
           const int n = (kt - s.t0) + (slot < 0 ? 0 : (slot >> 2));
-          for (; stat_waited <= n; ++stat_waited) B1_WAIT(W_STAT, bars + BAR_STAT + stat_waited % 3, (stat_waited / 3) & 1);
+          for (; stat_waited <= n; ++stat_waited) mbar_wait(bars + BAR_STAT + stat_waited % 3, (stat_waited / 3) & 1);
           const float* st = sStat + (n % 3) * 2 * kTile;
           const uint32_t tb = trow + S::COL_U + 64 * wg;           // this group's score buffer
           const uint32_t ta = trow + S::COL_A + 32 * wg;           // ... and 16-bit operand buffer: P^T 0-15 | dS^T 16-31
@@ -666,14 +616,11 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             mbar_arrive_warp(bars + BAR_U_FREE + wg);
           };
           auto wait_operands_free = [&]() {
-            if (u >= 2) B1_WAIT(W_UFREE, bars + BAR_A_FREE + wg, ((u - 2) >> 1) & 1);
+            if (u >= 2) mbar_wait(bars + BAR_A_FREE + wg, ((u - 2) >> 1) & 1);
             tc_fence_after();
           };
-          B1_WAIT(W_SREADY, bars + BAR_S_READY + wg, (u >> 1) & 1);
+          mbar_wait(bars + BAR_S_READY + wg, (u >> 1) & 1);
           tc_fence_after();
-#ifdef SVAE_DEBUG_BUILD
-          const long long t_unit = tl_on ? clock64() : 0;
-#endif
           // One code path for band units (lane = key of the tile, columns = the slot's 32 queries) and the global unit
           // (lane = query of the tile, columns = the 32 keys of block 0): x = S * scale*log2e + col_a[col] + row_a,
           // P = exp2(x), dS = P * (dP * scale + col_b[col] + row_b); the statistics -lse*log2e / -delta*scale are the
@@ -701,7 +648,6 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             row_a = st[row];
             row_b = st[kTile + row];
           }
-          live = live && !B1_KNOCK(1);
           if (live) {
             uint32_t sv[32], dv[32];
             tmem_ld32(tb, sv);
@@ -732,23 +678,15 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             for (int e = 0; e < 16; ++e) pk[e] = dk[e] = 0u;
           }
           wait_operands_free();
-#ifdef SVAE_DEBUG_BUILD
-          if (tl_on) {
-            tl_acc[live ? 12 : 14] += clock64() - t_unit;
-            tl_acc[13] += live ? 1 : 0;
-          }
-#endif
           if (!is_g) {
-            if (!B1_KNOCK(128)) {
-              tmem_st16(ta, pk);
-              tmem_st16(ta + 16, dk);
-            }
+            tmem_st16(ta, pk);
+            tmem_st16(ta + 16, dk);
             // dS^T row of this key -> staging tile (the dQ MMAs of the previous group must have read it)
-            if (grp >= 1) B1_WAIT(W_DSFREE, bars + BAR_DS_FREE, (grp - 1) & 1);
+            if (grp >= 1) mbar_wait(bars + BAR_DS_FREE, (grp - 1) & 1);
             uint8_t* half = sDS + ((slot & 3) >> 1) * S::TILE;
 #pragma unroll
             for (int ch = 0; ch < 4; ++ch)
-              if (!B1_KNOCK(128)) *reinterpret_cast<uint4*>(half + swz_off<128>(row, (slot & 1) * 4 + ch)) =
+              *reinterpret_cast<uint4*>(half + swz_off<128>(row, (slot & 1) * 4 + ch)) =
                   make_uint4(dk[4 * ch], dk[4 * ch + 1], dk[4 * ch + 2], dk[4 * ch + 3]);
             if (last_y) {                               // slots of the group that do not exist contribute nothing
               for (int sp = (slot & 3) + 1; sp < 4; ++sp) {
@@ -760,25 +698,17 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
             }
           } else {
             tmem_st16(ta, dk);                          // A operand of dQ X += dS_g K_0
-            if (gt >= 1) B1_WAIT(W_DSFREE, bars + BAR_G_FREE, (gt - 1) & 1);
+            if (gt >= 1) mbar_wait(bars + BAR_G_FREE, (gt - 1) & 1);
 #pragma unroll
             for (int ch = 0; ch < 4; ++ch) {            // row of [P_g (64 B) | dS_g (64 B)]
               *reinterpret_cast<uint4*>(sG + swz_off<128>(row, ch)) = make_uint4(pk[4 * ch], pk[4 * ch + 1], pk[4 * ch + 2], pk[4 * ch + 3]);
               *reinterpret_cast<uint4*>(sG + swz_off<128>(row, 4 + ch)) = make_uint4(dk[4 * ch], dk[4 * ch + 1], dk[4 * ch + 2], dk[4 * ch + 3]);
             }
           }
-#ifdef SVAE_DEBUG_BUILD
-          const long long t_tail = tl_on ? clock64() : 0;
-#endif
-          if (!B1_KNOCK(128)) {
-            fence_proxy_async();                        // staging tiles are read by the tensor core (async proxy)
-            tmem_wait_st();
-          }
+          fence_proxy_async();                          // staging tiles are read by the tensor core (async proxy)
+          tmem_wait_st();
           tc_fence_before();
           mbar_arrive_warp(bars + BAR_P_READY + wg);
-#ifdef SVAE_DEBUG_BUILD
-          if (tl_on) tl_acc[15] += clock64() - t_tail;
-#endif
           if (slot >= 0) mbar_arrive_warp(bars + (slot < 4 ? BAR_GRPX_READY : BAR_GRPY_READY));
         }
       }
@@ -786,14 +716,6 @@ attn_bwd1_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     }
   }
 
-#ifdef SVAE_DEBUG_BUILD
-  if (p.timeline && lane == 0) {
-    long long* tl = p.timeline + ((int64_t)blockIdx.x * 16 + warp) * 16;
-    for (int i = 0; i < 16; ++i) tl[i] = tl_acc[i];
-    tl[10] = clock64() - tl_start;
-    tl[11] = range_hi - range_lo;
-  }
-#endif
   tc_fence_before();
   __syncthreads();
   if (warp == 15) tmem_dealloc<512>(tmem_base);
@@ -871,12 +793,6 @@ static int launch_bwd1(const svae_attn_desc* d, const void* q, const void* k, co
   p.num_ctas = b1_num_ctas(p.num_tiles);
   p.maxseg = band.cls ? b1_maxseg(B * H, p.T, p.num_tiles, p.num_ctas) : 1;
   p.scale = d->scale; p.scale_log2 = d->scale * kLog2e;
-  p.timeline = nullptr;
-  p.knock = 0;
-#ifdef SVAE_DEBUG_BUILD
-  p.timeline = g_b1_timeline;
-  p.knock = g_b1_knock;
-#endif
 
   const CUtensorMapDataType dt = Elem<T>::tm;
   CUtensorMap tQ, tDO, tK, tV, tK32, tV32, tDQ, tDK, tDV;
@@ -915,10 +831,3 @@ int bwd1(const svae_attn_desc* d, const void* q, const void* k, const void* v, c
 
 }  // namespace sm100
 }  // namespace svae
-
-#ifdef SVAE_DEBUG_BUILD
-extern "C" __attribute__((visibility("default"))) void svae_debug_set_b1_timeline(long long* timeline) {
-  svae::sm100::g_b1_timeline = timeline;
-}
-extern "C" __attribute__((visibility("default"))) void svae_debug_set_b1_knock(int mask) { svae::sm100::g_b1_knock = mask; }
-#endif

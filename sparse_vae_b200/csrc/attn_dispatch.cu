@@ -14,9 +14,9 @@ int exact_bwd(const svae_attn_desc*, const void*, const void*, const void*, cons
 
 namespace sm100 {
 
-int fwd(const svae_attn_desc*, const void*, const void*, const void*, const float*, void*, float*, float*, long long*, cudaStream_t);
+int fwd(const svae_attn_desc*, const void*, const void*, const void*, const float*, void*, float*, float*, cudaStream_t);
 bool fwd_persist_supported(const svae_attn_desc*);
-int fwd_persist(const svae_attn_desc*, const void*, const void*, const void*, const float*, void*, float*, long long*, cudaStream_t);
+int fwd_persist(const svae_attn_desc*, const void*, const void*, const void*, const float*, void*, float*, cudaStream_t);
 size_t bwd_workspace(const svae_attn_desc*);
 bool bwd_supported(const svae_attn_desc*);
 bool bwd1_supported(const svae_attn_desc*);
@@ -159,7 +159,7 @@ extern "C" int svae_attn_fwd_slots(const svae_attn_desc* d) {
 }
 
 static int attn_fwd_impl(const svae_attn_desc* d, const void* q, const void* k, const void* v, const float* kpm,
-                         void* out, float* lse, float* s_dump, long long* timeline, void* stream) {
+                         void* out, float* lse, float* s_dump, void* stream) {
   int rc = validate(d, false);
   if (rc) return rc;
   SVAE_REQUIRE(q && k && v && out && lse, SVAE_ERR_INVALID, "svae_attn_fwd: null tensor pointer");
@@ -174,19 +174,20 @@ static int attn_fwd_impl(const svae_attn_desc* d, const void* q, const void* k, 
   // persistent warp-specialised kernel (69 us vs 104 us at the C2 shape): what the host wrapper asks for whenever the
   // geometry fits (<= 8 key slots); wider windows and score dumps take the one-CTA-per-tile kernel
   if (!s_dump && (d->flags & SVAE_ATTN_PERSISTENT) && sm100::fwd_persist_supported(d))
-    return sm100::fwd_persist(d, q, k, v, kpm, out, lse, timeline, st);
-  return sm100::fwd(d, q, k, v, kpm, out, lse, s_dump, timeline, st);
+    return sm100::fwd_persist(d, q, k, v, kpm, out, lse, st);
+  return sm100::fwd(d, q, k, v, kpm, out, lse, s_dump, st);
 }
 
 extern "C" int svae_attn_fwd(const svae_attn_desc* d, const void* q, const void* k, const void* v, const float* kpm,
                              void* out, float* lse, void* stream) {
-  return attn_fwd_impl(d, q, k, v, kpm, out, lse, nullptr, nullptr, stream);
+  return attn_fwd_impl(d, q, k, v, kpm, out, lse, nullptr, stream);
 }
 
 extern "C" int svae_attn_fwd_debug(const svae_attn_desc* d, const void* q, const void* k, const void* v,
                                    const float* kpm, void* out, float* lse, float* s_dump, long long* timeline,
                                    void* stream) {
-  return attn_fwd_impl(d, q, k, v, kpm, out, lse, s_dump, timeline, stream);
+  SVAE_REQUIRE(timeline == nullptr, SVAE_ERR_UNSUPPORTED, "svae_attn_fwd_debug: timeline is not supported, pass NULL");
+  return attn_fwd_impl(d, q, k, v, kpm, out, lse, s_dump, stream);
 }
 
 extern "C" size_t svae_attn_bwd_workspace_bytes(const svae_attn_desc* d) {

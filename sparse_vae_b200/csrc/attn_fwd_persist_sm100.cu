@@ -67,14 +67,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
   const TileGeom g = p.g;
   const int ns = g.nslots;
   const int nt = (num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;     // tiles of this CTA
-  if (p.timeline && threadIdx.x == 0) {          // debug: CTA start (role 1 of its first tile): clock, globaltimer, SM id
-    long long* tl = p.timeline + ((int64_t)blockIdx.x * 5 + 1) * 8;
-    unsigned smid;
-    unsigned long long gt;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    tl[0] = clock64(); tl[1] = (long long)gt; tl[2] = smid;
-  }
 
   if (threadIdx.x == 0) {
     for (int k = 0; k < 2; ++k) {
@@ -101,9 +93,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
     const int bh = id / tiles_per_seq;
     h = bh % p.H;
     b = bh / p.H;
-  };
-  auto tl_ptr = [&](int i, int role) -> long long* {
-    return (p.timeline && lane == 0) ? p.timeline + (((int64_t)blockIdx.x + (int64_t)i * gridDim.x) * 5 + role) * 8 : nullptr;
   };
   const uint32_t idesc_pv = make_idesc(kTile, DH, Elem<T>::fmt, 0, 1);
   // O (+)= P_j V_j for slots j = first, first + 2, ... of the tile in ring slot k
@@ -149,17 +138,9 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       const uint32_t idesc_s = make_idesc(kTile, ns * kBlock, Elem<T>::fmt, 0, 0);
       for (int i = 0; i < nt; ++i) {
         const int k = i & 1, n = i >> 1;
-        long long* tl = tl_ptr(i, 4);
-        if (tl) tl[0] = clock64();
         mbar_wait(qk_full + k, n & 1);
-        if (tl) tl[1] = clock64();
         if (i >= 2) mbar_wait(tmem_free + k, (n - 1) & 1);
-        if (i == 1 && p.stagger_cycles > 0) {    // start the second softmax group out of phase with the first
-          const long long t0 = clock64();
-          while (clock64() - t0 < p.stagger_cycles) {}
-        }
         tc_fence_after();
-        if (tl) tl[2] = clock64();
         const uint32_t q_addr = smem_u32(smem + S::OFF_Q + k * S::Q_BYTES);
         const uint32_t k_addr = smem_u32(smem + S::OFF_K + k * S::KV_BYTES);
 #pragma unroll
@@ -168,23 +149,18 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
                    make_smem_desc(k_addr + ks * 32, 16, 8 * ROWB, ROWB), idesc_s, ks > 0 ? 1u : 0u);
         tc_commit_w(s_ready + k);
         tc_commit_w(qk_free + k);
-        if (tl) tl[3] = clock64();
       }
     } else {
       // ---- warp 14: even-slot half of O(i) = P V, warp 15: odd-slot half
       const int first = warp - 14;
       for (int i = 0; i < nt; ++i) {
         const int k = i & 1, n = i >> 1;
-        long long* tl = first == 0 ? tl_ptr(i, 4) : nullptr;
-        if (tl) tl[4] = clock64();
         mbar_wait(p_ready + k, n & 1);
         mbar_wait(v_full + k, n & 1);
         tc_fence_after();
-        if (tl) tl[5] = clock64();
         issue_pv_chain(k, first, first ? S::O2_COL : S::O_COL);
         tc_commit_w(o_ready + k);
         tc_commit_w(v_free + k);
-        if (tl) tl[6] = clock64();
       }
     }
   } else if (warp >= 8) {
@@ -200,11 +176,8 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       const uint32_t trow = tmem_base + 256 * k + ((uint32_t)(w * 32) << 16);
       uint8_t* sOst = smem + S::OFF_OST + k * S::Q_BYTES;
       const float* sInv = reinterpret_cast<const float*>(smem + S::OFF_INV) + k * kTile;
-      long long* tl = (w == 0) ? tl_ptr(i, 3) : nullptr;
-      if (tl) tl[0] = clock64();
       mbar_wait(o_ready + k, n & 1);
       tc_fence_after();
-      if (tl) tl[1] = clock64();
       const float inv = sInv[row];             // written before the group's p_ready arrival (ordered through the MMA warp)
       uint32_t oa[32], ob[32];
       uint32_t pk[DH / 2];
@@ -222,7 +195,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
           pk[half * 16 + (c >> 1)] = Elem<T>::pack((__uint_as_float(oa[c]) + __uint_as_float(ob[c])) * inv,
                                                    (__uint_as_float(oa[c + 1]) + __uint_as_float(ob[c + 1])) * inv);
       }
-      if (tl) tl[2] = clock64();
 #pragma unroll
       for (int ch = 0; ch < DH / 8; ++ch)
         *reinterpret_cast<uint4*>(sOst + swz_off<ROWB>(row, ch)) = make_uint4(pk[4 * ch], pk[4 * ch + 1], pk[4 * ch + 2], pk[4 * ch + 3]);
@@ -234,7 +206,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
         asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");    // the OTHER staging tile has been read
       }
       named_bar_sync(3, 128);                  // nobody writes the other staging tile before its store has read it
-      if (tl) tl[3] = clock64();
     }
     if (tid_g == 0) tma_store_wait_all();
   } else {
@@ -253,10 +224,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
     const int first = g.cls + w;
     const int kdiag = g.causal ? g.left - 1 : -1;
 
-    // Ping-pong between the two groups (named barriers 4 / 5, 128 waiting + 128 arriving threads): the MUFU-bound
-    // exp pass of one group never overlaps the other's, which keeps the groups in antiphase -- one runs its
-    // CUDA-core softmax while the other waits for / feeds the tensor pipe.
-    if (p.stagger_cycles >= 0 && grp == 1) named_bar_arrive(4, 256);
     for (int i = grp; i < nt; i += 2) {
       const int n = i >> 1;
       int t, h, b;
@@ -291,14 +258,11 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
 #pragma unroll
       for (int kk = 0; kk < 4; ++kk) lv[kk] = kk < nlb && r < g.nb && slot_valid(first + kk);
 
-      long long* tl = (w == 0) ? tl_ptr(i, 0) : nullptr;
-      if (tl) tl[0] = clock64();
       mbar_wait(s_ready + grp, n & 1);
       tc_fence_after();
-      if (tl) tl[1] = clock64();
       // Both passes are ROLLED loops over the block-row's live slots (k = 0: global block, k = 1..4: band slot
       // first + k - 1), re-reading the scores from TMEM in pass 2: tcgen05.ld is cheap (~53 cycles per 4 KB per SMSP,
-      // tests/pipe_bench.py) while ~1.5 k instructions of straight-line code per tile do not fit the instruction
+      // profiles/r01b_pipe_bench.log) while ~1.5 k instructions of straight-line code per tile do not fit the instruction
       // cache next to the other warps' streams (13 % `no_inst` stalls in profiles/r01b_persist_hot_sass.txt).
       float m = -INFINITY, l0 = 0.f, l1 = 0.f;
       const bool g_diag = g.causal && g.cls && r == 0 && lg;      // block-row 0: the global block IS the diagonal
@@ -318,11 +282,9 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       }
       if (!has_kpm) m *= p.scale_log2;        // scale > 0: max commutes with the scaling
       const float neg_m = (m == -INFINITY) ? 0.f : -m;
-      if (tl) tl[2] = clock64();
 
       // ---- pass 2: P = exp2(s * scale_log2 + mask - m), written over S as packed 16-bit.  Slots are visited in
       //      increasing column order, so P_j (columns 16 j ..) only ever overwrites scores that were already consumed.
-      if (p.stagger_cycles >= 0) named_bar_sync(4 + grp, 256);
       uint32_t pk[16];
 #pragma unroll 1
       for (int k = 0; k < 5; ++k) {
@@ -335,7 +297,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
         slot_exp_pack<T>(v, pk, l0, l1, has_kpm, sKpm + j * kBlock, p.scale_log2, neg_m);
         tmem_st16(trow + 16 * j, pk);
       }
-      if (p.stagger_cycles >= 0) named_bar_arrive(4 + (grp ^ 1), 256);
 #pragma unroll
       for (int c = 0; c < 16; ++c) pk[c] = 0u;
       uint32_t live_mask = lg ? 1u : 0u;
@@ -348,7 +309,6 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       tmem_wait_st();
       tc_fence_before();
       mbar_arrive(p_ready + grp);
-      if (tl) tl[3] = clock64();
       if (qpos < p.L) p.lse[((int64_t)b * p.H + h) * p.L + qpos] = (m + log2f(l)) * kLn2;
     }
   }
@@ -356,17 +316,11 @@ attn_fwd_persist_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
   tc_fence_before();
   __syncthreads();
   if (warp == 15) tmem_dealloc<512>(tmem_base);
-  if (p.timeline && threadIdx.x == 0) {          // debug: CTA end (role 2 of its first tile)
-    long long* tl = p.timeline + ((int64_t)blockIdx.x * 5 + 2) * 8;
-    unsigned long long gt;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    tl[0] = clock64(); tl[1] = (long long)gt;
-  }
 }
 
 template <typename T, int DH>
 static int launch_fwd_persist(const svae_attn_desc* d, const TileGeom& g, const void* q, const void* k, const void* v,
-                              const float* kpm, void* out, float* lse, long long* timeline, cudaStream_t st) {
+                              const float* kpm, void* out, float* lse, cudaStream_t st) {
   using S = FwdPSmem<DH>;
   CUtensorMap tmQ, tmK, tmV, tmKb, tmVb, tmO;
   int rc;
@@ -378,10 +332,9 @@ static int launch_fwd_persist(const svae_attn_desc* d, const TileGeom& g, const 
   if ((rc = encode_tmap(&tmVb, Elem<T>::tm, v, DH, d->seq_len, d->heads, d->batch, d->v_stride, band_rows))) return rc;
   if ((rc = encode_tmap(&tmO, Elem<T>::tm, out, DH, d->seq_len, d->heads, d->batch, d->o_stride, kTile))) return rc;
   FwdParams p;
-  p.kpm = kpm; p.lse = lse; p.s_dump = nullptr; p.timeline = timeline;
+  p.kpm = kpm; p.lse = lse; p.s_dump = nullptr;
   p.L = d->seq_len; p.H = d->heads; p.g = g;
   p.scale_log2 = d->scale * kLog2e;
-  p.stagger_cycles = -1;                       // < 0: no ping-pong between the softmax groups (measured faster)
   auto kern = attn_fwd_persist_sm100_kernel<T, DH>;
   const int sm_count = sm_count_of_current_device();
   SVAE_CONFIGURE_SMEM(kern, S::DYN_BYTES);
@@ -402,13 +355,13 @@ bool fwd_persist_supported(const svae_attn_desc* d) {
 }
 
 int fwd_persist(const svae_attn_desc* d, const void* q, const void* k, const void* v, const float* kpm, void* out,
-                float* lse, long long* timeline, cudaStream_t st) {
+                float* lse, cudaStream_t st) {
   const TileGeom g = make_geom(d->window_size, d->causal, d->include_cls, d->seq_len / d->block_size);
   if (d->dtype == SVAE_DTYPE_BF16)
-    return d->head_dim == 64 ? launch_fwd_persist<__nv_bfloat16, 64>(d, g, q, k, v, kpm, out, lse, timeline, st)
-                             : launch_fwd_persist<__nv_bfloat16, 32>(d, g, q, k, v, kpm, out, lse, timeline, st);
-  return d->head_dim == 64 ? launch_fwd_persist<__half, 64>(d, g, q, k, v, kpm, out, lse, timeline, st)
-                           : launch_fwd_persist<__half, 32>(d, g, q, k, v, kpm, out, lse, timeline, st);
+    return d->head_dim == 64 ? launch_fwd_persist<__nv_bfloat16, 64>(d, g, q, k, v, kpm, out, lse, st)
+                             : launch_fwd_persist<__nv_bfloat16, 32>(d, g, q, k, v, kpm, out, lse, st);
+  return d->head_dim == 64 ? launch_fwd_persist<__half, 64>(d, g, q, k, v, kpm, out, lse, st)
+                           : launch_fwd_persist<__half, 32>(d, g, q, k, v, kpm, out, lse, st);
 }
 
 }  // namespace sm100

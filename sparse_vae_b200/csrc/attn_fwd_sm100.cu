@@ -74,11 +74,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   const int ns = g.nslots;
   const int r0 = 4 * t;
   const int band_lo = r0 - (g.left - 1);
-  long long* tl = nullptr;
-  if (p.timeline && lane == 0)
-    tl = p.timeline + ((((int64_t)b * gridDim.y + h) * gridDim.x + t) * 5 + warp) * 8;
-  auto stamp = [&](int k) { if (tl) tl[k] = clock64(); };
-  stamp(0);
 
   auto slot_block = [&](int j) { return (g.cls && j == 0) ? 0 : band_lo + j - g.cls; };
   // a slot carries keys the tile may attend: inside the sequence and not a duplicate of the global block.
@@ -112,7 +107,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  stamp(1);
 
   const uint32_t v_addr = smem_u32(sV);
   const uint32_t idesc_pv = make_idesc(kTile, DH, Elem<T>::fmt, 0, 1);
@@ -141,12 +135,10 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     tma_load_4d_w(sV + g.cls * S::SLOT_BYTES, &tmVband, bar_v, 0, band_lo * kBlock, h, b);
     if (band_slots > 8) tma_load_4d_w(sV + (g.cls + 8) * S::SLOT_BYTES, &tmVband2, bar_v, 0, (band_lo + 8) * kBlock, h, b);
     if (g.cls) tma_load_4d_w(sV, &tmV, bar_v, 0, 0, h, b);
-    stamp(2);
 
     // ---- S = Q K^T : M = 128, N = 32*ns (split at 256), K = DH in steps of 16
     mbar_wait(bar_qk, 0);
     tc_fence_after();
-    stamp(3);
     const uint32_t q_addr = smem_u32(sQ), k_addr = smem_u32(sK);
     const int ntot = ns * kBlock;
     for (int n0 = 0; n0 < ntot; n0 += 256) {
@@ -160,23 +152,13 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       }
     }
     tc_commit_w(bar_s);
-    stamp(4);
 
     // ---- O = P V, chain A (every second slot when a softmax warp issues the other half)
     mbar_wait(bar_p, 0);
     mbar_wait(bar_v, 0);
     tc_fence_after();
-    stamp(5);
     issue_pv_chain(0, kTwoChains ? 2 : 1, S::O_COL);
     tc_commit_w(bar_o);
-    stamp(6);
-    if (tl) {
-      unsigned smid;
-      asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-      unsigned long long gt;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-      tl[7] = (long long)((gt << 8) | (smid & 255));
-    }
   } else {
     // ================= softmax + epilogue warps: warp w <-> block-row r0 + w <-> TMEM lanes 32w.. =================
     const int r = r0 + warp;
@@ -207,7 +189,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 
     mbar_wait(bar_s, 0);
     tc_fence_after();
-    stamp(2);
 
     if (p.s_dump) {   // debug only
       for (int j = 0; j < ns; ++j) {
@@ -237,7 +218,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       }
       if (!has_kpm) m *= p.scale_log2;
       neg_m = (m == -INFINITY) ? 0.f : -m;
-      stamp(3);
       for (int j = 0; j < ns; ++j) {
         uint32_t pk[16];
         if (slot_live(j)) {
@@ -257,7 +237,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     tmem_wait_st();
     tc_fence_before();
     mbar_arrive(bar_p);
-    stamp(4);
 
     if (kTwoChains && warp == 0) {
       // ---- O2 = P V, chain B (odd slots), issued by this warp while it would otherwise idle until O is ready
@@ -273,7 +252,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     const float inv = 1.0f / l;     // l == 0 (row with every key masked) -> NaN, like the reference softmax
     mbar_wait(bar_o, 0);
     tc_fence_after();
-    stamp(5);
 #pragma unroll
     for (int half = 0; half < DH / 32; ++half) {
       uint32_t v[32];
@@ -304,7 +282,6 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       tma_store_commit();
       tma_store_wait_read();
     }
-    stamp(6);
   }
 
   tc_fence_before();
@@ -314,7 +291,7 @@ attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 
 template <typename T, int DH, int NSMAX>
 static int launch_fwd(const svae_attn_desc* d, const TileGeom& g, const void* q, const void* k, const void* v,
-                      const float* kpm, void* out, float* lse, float* s_dump, long long* timeline, cudaStream_t st) {
+                      const float* kpm, void* out, float* lse, float* s_dump, cudaStream_t st) {
   using S = FwdSmem<DH, NSMAX>;
   CUtensorMap tmQ, tmK, tmV, tmKb, tmVb, tmKb2, tmVb2, tmO;
   int rc;
@@ -329,10 +306,9 @@ static int launch_fwd(const svae_attn_desc* d, const TileGeom& g, const void* q,
   if ((rc = encode_tmap(&tmVb2, Elem<T>::tm, v, DH, d->seq_len, d->heads, d->batch, d->v_stride, band2_rows))) return rc;
   if ((rc = encode_tmap(&tmO, Elem<T>::tm, out, DH, d->seq_len, d->heads, d->batch, d->o_stride, kTile))) return rc;
   FwdParams p;
-  p.kpm = kpm; p.lse = lse; p.s_dump = s_dump; p.timeline = timeline;
+  p.kpm = kpm; p.lse = lse; p.s_dump = s_dump;
   p.L = d->seq_len; p.H = d->heads; p.g = g;
   p.scale_log2 = d->scale * kLog2e;
-  p.stagger_cycles = 0;
   auto kern = attn_fwd_sm100_kernel<T, DH, NSMAX>;
   SVAE_CONFIGURE_SMEM(kern, S::DYN_BYTES);
   dim3 grid((d->seq_len + kTile - 1) / kTile, d->heads, d->batch);
@@ -345,15 +321,15 @@ static int launch_fwd(const svae_attn_desc* d, const TileGeom& g, const void* q,
 int fwd_max_slots() { return 14; }
 
 int fwd(const svae_attn_desc* d, const void* q, const void* k, const void* v, const float* kpm, void* out, float* lse,
-        float* s_dump, long long* timeline, cudaStream_t st) {
+        float* s_dump, cudaStream_t st) {
   const TileGeom g = make_geom(d->window_size, d->causal, d->include_cls, d->seq_len / d->block_size);
   SVAE_REQUIRE(g.nslots <= 14, SVAE_ERR_UNSUPPORTED, "sm100 attention forward: %d key slots (window %d) exceed 14",
                g.nslots, d->window_size);
   SVAE_REQUIRE(d->scale > 0.f, SVAE_ERR_UNSUPPORTED, "sm100 attention forward: softmax scale must be positive");
   const bool small = g.nslots <= 8 && g.left + g.nsup <= 4;   // the register-resident softmax holds <= 4 band slots
 #define SVAE_FWD(T, DH)                                                                              \
-  return small ? launch_fwd<T, DH, 8>(d, g, q, k, v, kpm, out, lse, s_dump, timeline, st)            \
-               : launch_fwd<T, DH, 14>(d, g, q, k, v, kpm, out, lse, s_dump, timeline, st)
+  return small ? launch_fwd<T, DH, 8>(d, g, q, k, v, kpm, out, lse, s_dump, st)                      \
+               : launch_fwd<T, DH, 14>(d, g, q, k, v, kpm, out, lse, s_dump, st)
   if (d->dtype == SVAE_DTYPE_BF16) {
     if (d->head_dim == 64) { SVAE_FWD(__nv_bfloat16, 64); }
     if (d->head_dim == 32) { SVAE_FWD(__nv_bfloat16, 32); }

@@ -72,11 +72,9 @@ struct FwdParams {
   const float* kpm;     // [B, L] additive or null
   float* lse;           // [B, H, L]
   float* s_dump;        // debug: [B, H, L, nslots*32] raw scores, or null
-  long long* timeline;  // debug: [num_ctas, 5 warps, 8] clock64 stamps, or null
   int L, H;
   TileGeom g;
   float scale_log2;     // scale * log2(e)
-  int stagger_cycles;   // persistent kernel: delay of the second softmax group's first tile
 };
 
 struct BwdParams {
@@ -87,7 +85,6 @@ struct BwdParams {
   int L, H;
   TileGeom g;
   float scale, scale_log2;
-  long long* timeline;  // debug: [2 kernels][num_ctas][3 roles (warp 0, warp 3, MMA warp)][16] clock64 stamps, or null
 };
 
 // ---- per-slot CUDA-core work on one row's 32 scores held in registers --------------------------------------

@@ -258,9 +258,9 @@ __global__ void __launch_bounds__(kBnThreads) bottleneck_bwd_kernel(BnBwdArgs a)
 // (row r0 + j*R, d) is component j of call m of "thread" i*latent + d -- no division per element.  A lane owns TWO
 // adjacent features: 4-byte loads of the 16-bit inputs (8-byte for fp32), 8-byte stores -> every warp request is a
 // full 128 / 256-byte line.
-#ifndef SVAE_BN_VEC_BLOCKS
-#define SVAE_BN_VEC_BLOCKS 4      // resident blocks per SM the vectorised kernels are compiled for (register cap 64)
-#endif
+// Resident blocks per SM the vectorised kernels are compiled for (register cap 64); 3 / 5 / 6 blocks per SM were
+// slower (DESIGN.md section 4.4).
+constexpr int kBnVecBlocks = 4;
 template <typename T> struct Pair;
 template <> struct Pair<float> {
   __device__ static __forceinline__ float2 load(const float* p) { return *reinterpret_cast<const float2*>(p); }
@@ -284,7 +284,7 @@ template <> struct Pair<__half> {
 __device__ __forceinline__ float comp4(const float4& v, int j) { return j == 0 ? v.x : j == 1 ? v.y : j == 2 ? v.z : v.w; }
 
 template <typename T>
-__global__ void __launch_bounds__(kBnThreads, SVAE_BN_VEC_BLOCKS) bottleneck_fwd_vec_kernel(BnFwdArgs a) {
+__global__ void __launch_bounds__(kBnThreads, kBnVecBlocks) bottleneck_fwd_vec_kernel(BnFwdArgs a) {
   a.pp = resolve(a.pp);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int warps_per_block = kBnThreads / 32;
@@ -373,7 +373,7 @@ __global__ void __launch_bounds__(kBnThreads, SVAE_BN_VEC_BLOCKS) bottleneck_fwd
 }
 
 template <typename T>
-__global__ void __launch_bounds__(kBnThreads, SVAE_BN_VEC_BLOCKS) bottleneck_bwd_vec_kernel(BnBwdArgs a) {
+__global__ void __launch_bounds__(kBnThreads, kBnVecBlocks) bottleneck_bwd_vec_kernel(BnBwdArgs a) {
   a.pp = resolve(a.pp);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int warps_per_block = kBnThreads / 32;
@@ -444,11 +444,7 @@ static int make_plan(int64_t rows, int latent, uint64_t seed, uint64_t offset, i
   p->pp.T = T;
   p->pp.dev = nullptr;
   p->share = (T % latent == 0);
-#ifdef SVAE_BN_NO_VEC
-  p->vec = false;
-#else
   p->vec = p->share && latent % 2 == 0;
-#endif
   if (p->share) {
     int64_t R = T / latent;
     p->rows_per_T = R;

@@ -15,10 +15,6 @@
 
 #include "common.cuh"
 
-#ifndef SVAE_ROTARY_PIPELINE
-#define SVAE_ROTARY_PIPELINE 1
-#endif
-
 namespace svae {
 
 template <typename T> struct RotOps;
@@ -160,7 +156,6 @@ __global__ void __launch_bounds__(256) rotary_pair_kernel(const T* xa, const T* 
       if (row < rows) v = *reinterpret_cast<const Pack<T, 8>*>(p + row * in_ld + vec * 8);
       return v;
     };
-#if SVAE_ROTARY_PIPELINE
     Pack<T, 8> a0 = ld(xa, r), b0 = ld(xb, r), a1 = ld(xa, r + step), b1 = ld(xb, r + step);
     for (; r < rows; r += 2 * step) {
       const int64_t rn = r + 2 * step;
@@ -169,14 +164,6 @@ __global__ void __launch_bounds__(256) rotary_pair_kernel(const T* xa, const T* 
       if (r + step < rows) one(r + step, a1, b1);
       a0 = na0; b0 = nb0; a1 = na1; b1 = nb1;
     }
-#else
-    for (; r + step < rows; r += 2 * step) {
-      const Pack<T, 8> a0 = ld(xa, r), b0 = ld(xb, r), a1 = ld(xa, r + step), b1 = ld(xb, r + step);
-      one(r, a0, b0);
-      one(r + step, a1, b1);
-    }
-    if (r < rows) one(r, ld(xa, r), ld(xb, r));
-#endif
   }
   if constexpr (kSums) {
     const int64_t plane = (int64_t)gridDim.y * d;            // partial: [2][slabs][d]

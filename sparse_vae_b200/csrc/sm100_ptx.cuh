@@ -31,35 +31,13 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// SVAE_MBAR_MODE (experiments, tests/mbar_modes.sh): 0 = mbarrier.try_wait with the system-dependent suspend time,
-// 1 = mbarrier.test_wait (never suspends: pure polling), 2 = try_wait with a suspend-time hint of SVAE_MBAR_HINT_NS
-#ifndef SVAE_MBAR_MODE
-#define SVAE_MBAR_MODE 0
-#endif
-#ifndef SVAE_MBAR_HINT_NS
-#define SVAE_MBAR_HINT_NS 32
-#endif
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
-#if SVAE_MBAR_MODE == 1
-  asm volatile(
-      "{\n\t.reg .pred P;\n\tmbarrier.test_wait.parity.shared::cta.b64 P, [%1], %2;\n\tselp.u32 %0, 1, 0, P;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-#elif SVAE_MBAR_MODE == 2
-  asm volatile(
-      "{\n\t.reg .pred P;\n\tmbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, P;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)SVAE_MBAR_HINT_NS)
-      : "memory");
-#else
   asm volatile(
       "{\n\t.reg .pred P;\n\tmbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\tselp.u32 %0, 1, 0, P;\n\t}"
       : "=r"(ok)
       : "r"(smem_u32(bar)), "r"(parity)
       : "memory");
-#endif
   return ok != 0;
 }
 // Bounded wait: a protocol bug traps (-> CUDA error on the host) instead of hanging the GPU.  Kept inline and
@@ -68,7 +46,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   // try_wait suspends the thread for a hardware-defined interval by itself; the clock (expensive to read, and a
   // serialising instruction) is only consulted once a wait has lasted far longer than any legitimate one
 #pragma unroll 1
-  for (int i = 0; i < (SVAE_MBAR_MODE == 0 ? 4096 : 1 << 20); ++i)
+  for (int i = 0; i < 4096; ++i)
     if (mbar_try_wait(bar, parity)) return;
   const long long t0 = clock64();
   while (!mbar_try_wait(bar, parity)) {
@@ -244,7 +222,7 @@ __device__ __forceinline__ bool bar_red_or(int id, int nthreads, uint32_t pred) 
 // The `_w` wrappers are executed by ALL 32 lanes of a warp with warp-uniform operands; one lane is elected inside
 // the asm.  Issuing from an `if (lane == 0)` branch instead makes ptxas treat every operand as divergent and wrap
 // each UTCHMMA / UTMALDG in an ELECT + R2UR waterfall loop: measured 127 cycles per tcgen05.mma versus 75 here
-// (tests/mma_bench.py, profiles/README.md).
+// (profiles/README.md).
 __device__ __forceinline__ int warp_index() { return __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0); }
 
 __device__ __forceinline__ void mma_ss_w(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
