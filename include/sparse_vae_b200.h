@@ -200,6 +200,21 @@ SVAE_API int svae_xattn_bwd(const svae_xattn_desc* desc, const void* q, const vo
                    const void* dout, const float* lse, const float* key_padding_mask, void* dq, void* dk, void* dv,
                    void* stream);
 
+/* ---- dense CAUSAL self-attention with additive key padding (the non-sparse decoders in training; reference
+ * core/attention.py:83-100 with causal=True and a padding mask).  Uses svae_xattn_desc with num_queries == num_keys = L:
+ *   out[b,h,i,:] = softmax_{j <= i}(scale * q_i . k_j + key_padding_mask[b, j]) v_j ; lse: fp32 [batch, heads, L], natural log.
+ * Keys j > i never enter the sum.  key_padding_mask: additive fp32 [batch, L] or NULL.  16-bit, head_dim 64, any L >= 1;
+ * q/k/v/out/dout/dq/dk/dv 16-byte aligned with strides that are multiples of 8 elements.  Deterministic (no atomics),
+ * no host synchronisation. */
+SVAE_API int svae_causal_attn_supported(const svae_xattn_desc* desc);
+SVAE_API int svae_causal_attn_fwd(const svae_xattn_desc* desc, const void* q, const void* k, const void* v,
+                         const float* key_padding_mask, void* out, float* lse, void* stream);
+/* device scratch of the backward (fp32 rowsum(dO o O) per query); 0 when the desc is outside svae_causal_attn_supported */
+SVAE_API size_t svae_causal_attn_bwd_workspace_bytes(const svae_xattn_desc* desc);
+SVAE_API int svae_causal_attn_bwd(const svae_xattn_desc* desc, const void* q, const void* k, const void* v, const void* out,
+                         const void* dout, const float* lse, const float* key_padding_mask, void* dq, void* dk, void* dv,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- CUDA-graph variants (core/graph_step.py): a captured training step is replayed with NEW random numbers and NEW
  * optimizer scalars each time, so these read them from device memory the host refreshes before every replay.
  * philox_dev -> {seed, base offset} (uint64[2]); the `offset` argument is then the launch's fixed increment over the base

@@ -43,6 +43,7 @@ EXPORTS = (
     'svae_dropout_branch_grad', 'svae_bottleneck_fwd_g', 'svae_bottleneck_bwd_g', 'svae_residual_dropout_add_g',
     'svae_dropout_branch_grad_g', 'svae_radam_args_bytes', 'svae_radam_args', 'svae_radam_step_g',
     'svae_xattn_supported', 'svae_xattn_fwd', 'svae_xattn_bwd',
+    'svae_causal_attn_supported', 'svae_causal_attn_fwd', 'svae_causal_attn_bwd_workspace_bytes', 'svae_causal_attn_bwd',
     'svae_rotary_pair_workspace_floats', 'svae_rotary_pair', 'svae_embedding_bwd',
     'svae_gelu_supported', 'svae_gelu_fwd', 'svae_gelu_bwd_workspace_floats', 'svae_gelu_bwd_counters', 'svae_gelu_bwd',
     'svae_vocab_logprob_supported', 'svae_vocab_logprob',

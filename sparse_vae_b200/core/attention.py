@@ -23,7 +23,7 @@ from .layer_norm import LayerNorm
 from .gelu import GELU, ffn_forward
 from .linear import Linear, linear3, qkv_rotary
 from .padded_tensor import split_padding
-from . import cross_attention
+from . import causal_attention, cross_attention
 from .residual import residual_add, residual_dropout_add
 from .rotary_embedding import RotaryEmbedding
 from .sparse_attention import SparseAttention
@@ -169,6 +169,11 @@ class Attention(nn.Module):
         if sparse and self.key_cache is None:
             kpm = padding * -1e7 if padding is not None else None
             out = sparse(q, k, v, key_padding_mask=kpm, joint_grads=fused is not None)  # [B, H, L, Dh] over [B, L, H, Dh]
+        elif (N.FUSED_EXTRAS and self.causal and self.key_cache is None and padding is not None and padding.ndim == 2
+              and causal_attention.supported(q, k, v)):
+            # dense causal self-attention of a padded training batch (the non-sparse decoders): the tcgen05 kernels of
+            # csrc/causal_attn_sm100.cu instead of the explicit [B, H, L, L] form below; same additive -1e7 mask
+            out = causal_attention.causal_attention(q, k, v, padding * -1e7, joint_grads=fused is not None)
         elif (N.FUSED_EXTRAS and not self.causal and self.key_cache is None and (padding is None or padding.ndim == 2)
               and cross_attention.supported(q, k, v)):
             # the Perceiver encoder's learned queries (<= 64) over the whole sequence: K and V streamed once through
