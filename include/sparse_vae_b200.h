@@ -199,6 +199,22 @@ SVAE_API int svae_xattn_fwd(const svae_xattn_desc* desc, const void* q, const vo
 SVAE_API int svae_xattn_bwd(const svae_xattn_desc* desc, const void* q, const void* k, const void* v, const void* out,
                    const void* dout, const float* lse, const float* key_padding_mask, void* dq, void* dk, void* dv,
                    void* stream);
+/* The same with the key range split across key_splits CTAs per (batch, head) pair, for few pairs over long keys.  Split s
+ * owns a contiguous, balanced run of the 128-key tiles.  Forward: each split writes its normalised partial output in fp32
+ * to the workspace and a merge launch combines them per query row, in split order.  Backward: each split stores dK / dV
+ * of its own tiles and its partial dQ in fp32; a reduce launch sums the partials in split order into dq.  No atomics
+ * (bit-deterministic), no host synchronisation.  key_splits = 1 launches exactly what svae_xattn_fwd / _bwd launch.
+ * svae_xattn_key_splits: the library's choice (1 from 64 pairs on; otherwise about SMs / pairs, each split keeping a
+ * few tiles).  svae_xattn_workspace_bytes: device scratch for either direction, 0 for one split (0 as well for a
+ * count outside 1..key tiles, which the split entries reject). */
+SVAE_API int svae_xattn_key_splits(const svae_xattn_desc* desc);
+SVAE_API size_t svae_xattn_workspace_bytes(const svae_xattn_desc* desc, int key_splits);
+SVAE_API int svae_xattn_fwd_split(const svae_xattn_desc* desc, int key_splits, const void* q, const void* k, const void* v,
+                   const float* key_padding_mask, void* out, float* lse, void* workspace, size_t workspace_bytes,
+                   void* stream);
+SVAE_API int svae_xattn_bwd_split(const svae_xattn_desc* desc, int key_splits, const void* q, const void* k, const void* v,
+                   const void* out, const void* dout, const float* lse, const float* key_padding_mask, void* dq, void* dk,
+                   void* dv, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- dense CAUSAL self-attention with additive key padding (the non-sparse decoders in training; reference
  * core/attention.py:83-100 with causal=True and a padding mask).  Uses svae_xattn_desc with num_queries == num_keys = L:

@@ -42,7 +42,8 @@ EXPORTS = (
     'svae_residual_layernorm', 'svae_residual_add', 'svae_multi_tensor_cast', 'svae_residual_dropout_add',
     'svae_dropout_branch_grad', 'svae_bottleneck_fwd_g', 'svae_bottleneck_bwd_g', 'svae_residual_dropout_add_g',
     'svae_dropout_branch_grad_g', 'svae_radam_args_bytes', 'svae_radam_args', 'svae_radam_step_g',
-    'svae_xattn_supported', 'svae_xattn_fwd', 'svae_xattn_bwd',
+    'svae_xattn_supported', 'svae_xattn_fwd', 'svae_xattn_bwd', 'svae_xattn_key_splits', 'svae_xattn_workspace_bytes',
+    'svae_xattn_fwd_split', 'svae_xattn_bwd_split',
     'svae_causal_attn_supported', 'svae_causal_attn_fwd', 'svae_causal_attn_bwd_workspace_bytes', 'svae_causal_attn_bwd',
     'svae_rotary_pair_workspace_floats', 'svae_rotary_pair', 'svae_embedding_bwd',
     'svae_gelu_supported', 'svae_gelu_fwd', 'svae_gelu_bwd_workspace_floats', 'svae_gelu_bwd_counters', 'svae_gelu_bwd',

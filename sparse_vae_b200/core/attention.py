@@ -177,8 +177,9 @@ class Attention(nn.Module):
         elif (N.FUSED_EXTRAS and not self.causal and self.key_cache is None and (padding is None or padding.ndim == 2)
               and cross_attention.supported(q, k, v)):
             # the Perceiver encoder's learned queries (<= 64) over the whole sequence: K and V streamed once through
-            # the tcgen05 kernels of csrc/xattn_sm100.cu; the additive mask is the reference's float32 -1e7
-            out = cross_attention.cross_attention(q, k, v, None if padding is None else padding * -1e7)
+            # the tcgen05 kernels of csrc/xattn_sm100.cu, the keys split across CTAs when the batch has few (batch, head)
+            # pairs; the additive mask is the reference's float32 -1e7
+            out = cross_attention.cross_attention(q, k, v, None if padding is None else padding * -1e7, key_splits=None)
         elif (N.FUSED_EXTRAS and q.is_cuda and self.key_cache is None and q.ndim == 4
               and (padding is None or (padding.ndim == 2 and not self.causal))):
             # Dense attention of the Perceiver encoder (64 learned queries over the whole sequence) and of non-sparse

@@ -1,6 +1,9 @@
 """Dense attention of a few queries over a long key sequence on the sm_100a kernels (csrc/xattn_sm100.cu): the Perceiver
 encoder's learned-query layers -- 64 latents attending all L tokens (reference core/perceiver.py:16-50 through the dense
-branch of core/attention.py:83-100: softmax(q k^T / sqrt(d) - 1e7 * padding) v, non-causal)."""
+branch of core/attention.py:83-100: softmax(q k^T / sqrt(d) - 1e7 * padding) v, non-causal).
+
+With few (batch, head) pairs -- small batches of long samples -- the key range of each pair is split across CTAs and the
+partial results are merged by a second launch; the library picks the count (`default_key_splits()`)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -23,7 +26,9 @@ class XAttnDesc(C.Structure):
 
 
 _lib_ready = False
-MIN_PAIRS = 64        # (batch, head) pairs = CTAs below which the library kernel is faster
+# (batch, head) pairs the kernels need.  One CTA per pair fills the GPU from 64 pairs on; fewer pairs split their keys
+# across CTAs (svae_xattn_key_splits) instead of leaving the work to the library's attention.
+MIN_PAIRS = 1
 
 
 def _bind():
@@ -37,6 +42,14 @@ def _bind():
     N.lib.svae_xattn_fwd.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp]
     N.lib.svae_xattn_bwd.restype = C.c_int
     N.lib.svae_xattn_bwd.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    N.lib.svae_xattn_key_splits.restype = C.c_int
+    N.lib.svae_xattn_key_splits.argtypes = [dp]
+    N.lib.svae_xattn_workspace_bytes.restype = C.c_size_t
+    N.lib.svae_xattn_workspace_bytes.argtypes = [dp, C.c_int]
+    N.lib.svae_xattn_fwd_split.restype = C.c_int
+    N.lib.svae_xattn_fwd_split.argtypes = [dp, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
+    N.lib.svae_xattn_bwd_split.restype = C.c_int
+    N.lib.svae_xattn_bwd_split.argtypes = [dp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
     _lib_ready = True
 
 
@@ -54,17 +67,33 @@ def _blhd(B, H, L, Dh, like):
     return torch.empty(B, L, H, Dh, dtype=like.dtype, device=like.device).permute(0, 2, 1, 3)
 
 
+def _workspace(desc, key_splits, device):
+    """fp32 partials of the split launches (None for one split); torch.empty is legal inside a graph capture."""
+    n = N.lib.svae_xattn_workspace_bytes(C.byref(desc), key_splits)
+    return torch.empty(n, dtype=torch.uint8, device=device) if n else None
+
+
 class _CrossAttentionFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, q, k, v, kpm):
+    def forward(ctx, q, k, v, kpm, key_splits):
         q, k, v = _kernel_ready(q), _kernel_ready(k), _kernel_ready(v)
         B, H, nq, Dh = q.shape
         out = _blhd(B, H, nq, Dh, q)
         lse = torch.empty(B, H, nq, dtype=torch.float32, device=q.device)
         desc = _desc(q, k, v, out)
         with torch.cuda.device(q.device):
-            N.check(N.lib.svae_xattn_fwd(C.byref(desc), N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(kpm), N.ptr(out), N.ptr(lse),
-                                         N.current_stream(q.device)), 'svae_xattn_fwd')
+            if key_splits is None:
+                key_splits = N.lib.svae_xattn_key_splits(C.byref(desc))
+                N.check(min(key_splits, 0), 'svae_xattn_key_splits')
+            if key_splits == 1:
+                N.check(N.lib.svae_xattn_fwd(C.byref(desc), N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(kpm), N.ptr(out), N.ptr(lse),
+                                             N.current_stream(q.device)), 'svae_xattn_fwd')
+            else:
+                ws = _workspace(desc, key_splits, q.device)
+                N.check(N.lib.svae_xattn_fwd_split(C.byref(desc), key_splits, N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(kpm), N.ptr(out),
+                                                   N.ptr(lse), N.ptr(ws), 0 if ws is None else ws.numel(),
+                                                   N.current_stream(q.device)), 'svae_xattn_fwd_split')
+        ctx.key_splits = key_splits
         ctx.save_for_backward(q, k, v, out, lse, kpm)
         return out
 
@@ -78,10 +107,18 @@ class _CrossAttentionFn(torch.autograd.Function):
         dk, dv = _blhd(B, H, Lk, Dh, q), _blhd(B, H, Lk, Dh, q)
         desc = _desc(q, k, v, out)
         desc.do_stride, desc.dq_stride, desc.dk_stride, desc.dv_stride = _strides3(dout), _strides3(dq), _strides3(dk), _strides3(dv)
+        key_splits = ctx.key_splits
         with torch.cuda.device(q.device):
-            N.check(N.lib.svae_xattn_bwd(C.byref(desc), N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(out), N.ptr(dout), N.ptr(lse), N.ptr(kpm),
-                                         N.ptr(dq), N.ptr(dk), N.ptr(dv), N.current_stream(q.device)), 'svae_xattn_bwd')
-        return dq, dk, dv, None
+            if key_splits == 1:
+                N.check(N.lib.svae_xattn_bwd(C.byref(desc), N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(out), N.ptr(dout), N.ptr(lse),
+                                             N.ptr(kpm), N.ptr(dq), N.ptr(dk), N.ptr(dv), N.current_stream(q.device)), 'svae_xattn_bwd')
+            else:
+                ws = _workspace(desc, key_splits, q.device)
+                N.check(N.lib.svae_xattn_bwd_split(C.byref(desc), key_splits, N.ptr(q), N.ptr(k), N.ptr(v), N.ptr(out), N.ptr(dout),
+                                                   N.ptr(lse), N.ptr(kpm), N.ptr(dq), N.ptr(dk), N.ptr(dv), N.ptr(ws),
+                                                   0 if ws is None else ws.numel(), N.current_stream(q.device)),
+                        'svae_xattn_bwd_split')
+        return dq, dk, dv, None, None
 
 
 def _compute_dtype(q: Tensor, k: Tensor, v: Tensor):
@@ -93,19 +130,31 @@ def _compute_dtype(q: Tensor, k: Tensor, v: Tensor):
 
 
 def supported(q: Tensor, k: Tensor, v: Tensor) -> bool:
-    """16-bit CUDA tensors [B, H, nq <= 64, 64] against [B, H, Lk, 64]; worth it from a few hundred keys on.  One CTA
-    streams the keys of one (batch, head) pair, so the kernels need batch * heads >= 64 of them to fill the 148 SMs: the
-    long-context configuration (4 x 16384 tokens per GPU = 32 pairs) measured 239 / 194 us against the library's 142 / 196
-    and stays on `scaled_dot_product_attention` until the key range is split across CTAs."""
+    """16-bit CUDA tensors [B, H, nq <= 64, 64] against [B, H, Lk, 64]; worth it from a few hundred keys on.  Any number
+    of (batch, head) pairs: below 64 the key range of each pair is split across CTAs (`key_splits`)."""
     _bind()
     return (q.is_cuda and q.ndim == 4 and _compute_dtype(q, k, v) in (torch.bfloat16, torch.float16)
             and q.shape[-1] == 64 and k.shape[-1] == 64 and 1 <= q.shape[-2] <= 64 and k.shape[-2] >= 256
             and k.shape == v.shape and q.shape[:2] == k.shape[:2] and q.shape[0] * q.shape[1] >= MIN_PAIRS)
 
 
-def cross_attention(q: Tensor, k: Tensor, v: Tensor, key_padding_mask: Tensor = None) -> Tensor:
+def default_key_splits(q: Tensor, k: Tensor) -> int:
+    """The library's key split count for q [B, H, nq, 64] over k [B, H, Lk, 64] on q's device."""
+    _bind()
+    d = XAttnDesc()
+    d.batch, d.heads, d.num_queries, d.num_keys, d.head_dim = *q.shape[:3], k.shape[-2], q.shape[-1]
+    d.dtype, d.scale = N.DTYPE_BF16, float(q.shape[-1] ** -0.5)
+    with torch.cuda.device(q.device):
+        n = N.lib.svae_xattn_key_splits(C.byref(d))
+    N.check(min(n, 0), 'svae_xattn_key_splits')
+    return n
+
+
+def cross_attention(q: Tensor, k: Tensor, v: Tensor, key_padding_mask: Tensor = None, key_splits: int = 1) -> Tensor:
     """softmax(q k^T / sqrt(d) + key_padding_mask[:, None, None, :]) v; `key_padding_mask` additive fp32 [B, Lk] or None.
-    Returns [B, H, nq, Dh] as a view of [B, nq, H, Dh] memory (the caller's head merge is then a free view)."""
+    Returns [B, H, nq, Dh] as a view of [B, nq, H, Dh] memory (the caller's head merge is then a free view).
+    `key_splits`: CTAs per (batch, head) pair, each over a contiguous run of 128-key tiles (1..ceil(Lk / 128)); None
+    takes the library's choice.  Every count gives the same softmax up to fp32 rounding, each bit-deterministically."""
     _bind()
     if not q.is_cuda:
         raise ValueError("Only GPU devices are supported for now")
@@ -116,4 +165,4 @@ def cross_attention(q: Tensor, k: Tensor, v: Tensor, key_padding_mask: Tensor = 
     kpm = None
     if key_padding_mask is not None:
         kpm = key_padding_mask.detach().to(torch.float32).reshape(q.shape[0], k.shape[-2]).contiguous()
-    return _CrossAttentionFn.apply(q, k, v, kpm)
+    return _CrossAttentionFn.apply(q, k, v, kpm, key_splits)

@@ -12,7 +12,15 @@
 // S^T = K Q^T and dP^T = V dO^T (128 keys x nq queries) -> P^T, dS^T as 16-bit TMEM operands -> dV = P^T dO and
 // dK = dS^T Q stored per tile; dS^T also staged in shared memory for dQ += dS K, whose accumulator lives in TMEM for
 // the whole sequence.  No atomics: bit-deterministic.
+// Key splits (grid (B*H) x splits): below 64 (batch, head) pairs one CTA per pair leaves most SMs idle, so split s of a
+// pair takes a contiguous, balanced run of the 128-key tiles; only its TMA coordinates, key-mask staging and
+// "key >= Lk" test move.  With several splits the forward writes O_s / l_s, m_s and l_s in fp32 and
+// xattn_fwd_merge_kernel combines them in split order; the backward (merged lse, delta recomputed per CTA) stores dK / dV
+// of its own tiles and drains its partial dQ in fp32, which xattn_dq_reduce_kernel sums in split order.  One split
+// launches exactly the one-CTA-per-pair kernels above.
 // HBM roofline: forward reads K, V once; backward reads K, V and writes dK, dV once.
+#include <algorithm>
+
 #include "attn_sm100.cuh"
 
 namespace svae {
@@ -40,9 +48,18 @@ struct XParams {
   const float* kpm;     // [B, Lk] additive or null
   float* lse;           // [B, H, nq] natural log
   const float* delta;   // backward: unused (computed in the kernel)
+  float* part_o;        // key_splits > 1: [B*H][splits][nq][DH] the split's O_s / l_s, fp32
+  float* part_m;        // key_splits > 1: [B*H][splits][nq] the split's running maximum m_s (log2 domain)
+  float* part_l;        // key_splits > 1: [B*H][splits][nq] the split's row sum l_s relative to m_s
   int nq, Lk, H;
   float scale, scale_log2;
 };
+
+// key tiles [first, last) of split s of `splits` over nt tiles: contiguous, balanced to one tile, never empty (splits <= nt)
+__device__ __forceinline__ void x_split_tiles(int nt, int splits, int s, int& first, int& last) {
+  first = (int)((int64_t)s * nt / splits);
+  last = (int)((int64_t)(s + 1) * nt / splits);
+}
 
 template <typename T, int DH>
 __global__ void __launch_bounds__(kXThreads, 1)
@@ -65,7 +82,9 @@ xattn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
 
   const int warp = warp_index(), lane = threadIdx.x & 31;
   const int h = blockIdx.x % p.H, b = blockIdx.x / p.H;
-  const int nt = (p.Lk + kTile - 1) / kTile;
+  int t0, t1;                                          // this CTA's key tiles (all of them with one split)
+  x_split_tiles((p.Lk + kTile - 1) / kTile, gridDim.y, blockIdx.y, t0, t1);
+  const int nt = t1 - t0;
 
   if (threadIdx.x == 0) {
     mbar_init(q_full, 1);
@@ -92,9 +111,9 @@ xattn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       const int s = i % kXStages;
       if (i >= kXStages) mbar_wait(kv_free + s, ((i / kXStages) - 1) & 1);
       mbar_arrive_expect_tx_w(k_full + s, S::TILE);
-      tma_load_4d_w(smem + S::OFF_K + s * S::TILE, &tmK, k_full + s, 0, i * kTile, h, b);
+      tma_load_4d_w(smem + S::OFF_K + s * S::TILE, &tmK, k_full + s, 0, (t0 + i) * kTile, h, b);
       mbar_arrive_expect_tx_w(v_full + s, S::TILE);
-      tma_load_4d_w(smem + S::OFF_V + s * S::TILE, &tmV, v_full + s, 0, i * kTile, h, b);
+      tma_load_4d_w(smem + S::OFF_V + s * S::TILE, &tmV, v_full + s, 0, (t0 + i) * kTile, h, b);
     }
   } else if (warp == 5) {
     // ---- MMA issuer: S(0); then per tile  S(i+1) ; wait P(i) ; O += P(i) V(i)   (in-order pipe: S(i+1) overwrites the
@@ -138,7 +157,7 @@ xattn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     for (int i = 0; i < nt; ++i) {
       float* kp = sKpm + (i & 1) * kTile;
       {   // additive key terms of this tile: mask * log2(e), -inf beyond the sequence
-        const int key = i * kTile + (int)threadIdx.x;
+        const int key = (t0 + i) * kTile + (int)threadIdx.x;
         float kv = -INFINITY;
         if (key < p.Lk) kv = p.kpm ? p.kpm[(int64_t)b * p.Lk + key] * kLog2e : 0.f;
         kp[threadIdx.x] = kv;
@@ -219,33 +238,54 @@ xattn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       tc_fence_before();
       mbar_arrive(p_ready + (i & 1));
     }
-    // epilogue: O / l -> 16-bit -> swizzled staging (the Q tile) -> TMA store ; LSE
     mbar_wait(o_done, (nt - 1) & 1);
     tc_fence_after();
-    uint8_t* stage = smem + S::OFF_Q;
-    const float inv = 1.0f / l;
+    if (gridDim.y > 1) {
+      // epilogue of one split of several: O_s / l_s in fp32 and (m_s, l_s) for the merge launch.  A split whose keys are
+      // all -inf has l_s = 0: its O_s is written as 0 and the merge gives it weight 0.
+      const float inv = l > 0.f ? 1.0f / l : 0.f;
+      const int64_t slot = ((int64_t)blockIdx.x * gridDim.y + blockIdx.y) * p.nq + row;
 #pragma unroll
-    for (int half = 0; half < DH / 32; ++half) {
-      uint32_t o[32];
-      tmem_ld32(trow + COL_O + 32 * half, o);
-      tmem_wait_ld(o);
+      for (int half = 0; half < DH / 32; ++half) {
+        uint32_t o[32];
+        tmem_ld32(trow + COL_O + 32 * half, o);
+        tmem_wait_ld(o);
+        if (row < p.nq) {
+          float4* dst = reinterpret_cast<float4*>(p.part_o + slot * DH + 32 * half);
 #pragma unroll
-      for (int cq = 0; cq < 4; ++cq) {
-        uint4 w4;
-        w4.x = Elem<T>::pack(__uint_as_float(o[cq * 8 + 0]) * inv, __uint_as_float(o[cq * 8 + 1]) * inv);
-        w4.y = Elem<T>::pack(__uint_as_float(o[cq * 8 + 2]) * inv, __uint_as_float(o[cq * 8 + 3]) * inv);
-        w4.z = Elem<T>::pack(__uint_as_float(o[cq * 8 + 4]) * inv, __uint_as_float(o[cq * 8 + 5]) * inv);
-        w4.w = Elem<T>::pack(__uint_as_float(o[cq * 8 + 6]) * inv, __uint_as_float(o[cq * 8 + 7]) * inv);
-        *reinterpret_cast<uint4*>(stage + swz_off<ROWB>(row, half * 4 + cq)) = w4;
+          for (int e = 0; e < 8; ++e)
+            dst[e] = make_float4(__uint_as_float(o[4 * e]) * inv, __uint_as_float(o[4 * e + 1]) * inv,
+                                 __uint_as_float(o[4 * e + 2]) * inv, __uint_as_float(o[4 * e + 3]) * inv);
+        }
       }
-    }
-    if (row < p.nq) p.lse[((int64_t)b * p.H + h) * p.nq + row] = (m + log2f(l)) * kLn2;
-    fence_proxy_async();
-    named_bar_sync(1, 128);
-    if (threadIdx.x == 0) {
-      tma_store_4d(&tmO, stage, 0, 0, h, b);             // rows >= nq are outside the tensor: clipped
-      tma_store_commit();
-      tma_store_wait_all();
+      if (row < p.nq) { p.part_m[slot] = m; p.part_l[slot] = l; }
+    } else {
+      // epilogue: O / l -> 16-bit -> swizzled staging (the Q tile) -> TMA store ; LSE
+      uint8_t* stage = smem + S::OFF_Q;
+      const float inv = 1.0f / l;
+#pragma unroll
+      for (int half = 0; half < DH / 32; ++half) {
+        uint32_t o[32];
+        tmem_ld32(trow + COL_O + 32 * half, o);
+        tmem_wait_ld(o);
+#pragma unroll
+        for (int cq = 0; cq < 4; ++cq) {
+          uint4 w4;
+          w4.x = Elem<T>::pack(__uint_as_float(o[cq * 8 + 0]) * inv, __uint_as_float(o[cq * 8 + 1]) * inv);
+          w4.y = Elem<T>::pack(__uint_as_float(o[cq * 8 + 2]) * inv, __uint_as_float(o[cq * 8 + 3]) * inv);
+          w4.z = Elem<T>::pack(__uint_as_float(o[cq * 8 + 4]) * inv, __uint_as_float(o[cq * 8 + 5]) * inv);
+          w4.w = Elem<T>::pack(__uint_as_float(o[cq * 8 + 6]) * inv, __uint_as_float(o[cq * 8 + 7]) * inv);
+          *reinterpret_cast<uint4*>(stage + swz_off<ROWB>(row, half * 4 + cq)) = w4;
+        }
+      }
+      if (row < p.nq) p.lse[((int64_t)b * p.H + h) * p.nq + row] = (m + log2f(l)) * kLn2;
+      fence_proxy_async();
+      named_bar_sync(1, 128);
+      if (threadIdx.x == 0) {
+        tma_store_4d(&tmO, stage, 0, 0, h, b);             // rows >= nq are outside the tensor: clipped
+        tma_store_commit();
+        tma_store_wait_all();
+      }
     }
   }
   tc_fence_before();
@@ -253,14 +293,63 @@ xattn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
   if (warp == 5) tmem_dealloc<512>(tmem_base);
 }
 
+// grid (B * H, nq), DH threads (one per output column): per (pair, query row), over the splits in order,  M = max_s m_s,  w_s = l_s 2^(m_s - M),
+// out = sum_s w_s O_s / sum_s w_s,  lse = (M + log2 sum_s w_s) ln 2.  The split's (m_s, l_s) rather than its own lse
+// travel to the merge: next to the -1e7 key mask an fp32 lse is a number near -1e7 whose spacing is 1, so a split's
+// weight exp(lse_s - max lse) would be off by up to e^0.5, while m_s - M is exact there.
+template <typename T, int DH>
+__global__ void __launch_bounds__(DH)
+xattn_fwd_merge_kernel(const float* __restrict__ part_o, const float* __restrict__ part_m, const float* __restrict__ part_l,
+                       T* __restrict__ out, float* __restrict__ lse, int64_t os0, int64_t os1, int64_t os2, int H, int nq,
+                       int splits) {
+  const int pair = blockIdx.x, row = blockIdx.y, c = threadIdx.x, b = pair / H, h = pair - b * H;
+  const int64_t base = (int64_t)pair * splits;
+  float M = -INFINITY;
+  for (int s = 0; s < splits; ++s) M = fmaxf(M, part_m[(base + s) * nq + row]);
+  float L = 0.f, O = 0.f;
+  for (int s = 0; s < splits; ++s) {
+    const int64_t slot = (base + s) * nq + row;
+    const float ms = part_m[slot];
+    const float w = ms == -INFINITY ? 0.f : part_l[slot] * exp2f(ms - M);         // splits without a finite key: 0
+    L += w;
+    O = fmaf(w, part_o[slot * DH + c], O);
+  }
+  out[b * os0 + h * os1 + row * os2 + c] = from_f32<T>(O / L);     // no finite key at all: 0 / 0, as with one split
+  if (c == 0) lse[(int64_t)pair * nq + row] = (M + log2f(L)) * kLn2;
+}
+
 bool xattn_supported(const svae_xattn_desc* d) {
   if (d->dtype != SVAE_DTYPE_BF16 && d->dtype != SVAE_DTYPE_F16) return false;
   return d->head_dim == 64 && d->num_queries >= 1 && d->num_queries <= 128 && d->num_keys >= 1 && d->scale > 0.f;
 }
 
+int xattn_key_tiles(const svae_xattn_desc* d) { return (d->num_keys + kTile - 1) / kTile; }
+
+// The library's key split count.  One CTA per (batch, head) pair streams all keys of the pair; from kXMinPairs pairs on
+// that fills the GPU well enough (and those shapes keep exactly the one-split launch).  Below it each pair gets about
+// SMs / pairs CTAs (both kernels hold 512 TMEM columns: one CTA per SM, one wave), but every split keeps at least
+// kXMinSplitTiles key tiles.  Measured on a B200 (1000 W, 148 SMs) at 16 x 4096 tokens, 8 heads: the forward takes 66 us
+// with one split (32 tiles per CTA), 116 us with 16 (2 tiles per CTA) and 168 us with 32 -- a CTA's fixed work (TMEM
+// allocation, Q load, pipeline fill, epilogue) costs about two tiles, so splits shorter than ~8 tiles mostly pay for it.
+constexpr int kXMinPairs = 64;
+constexpr int kXMinSplitTiles = 8;
+
+int xattn_key_splits(const svae_xattn_desc* d) {
+  const int64_t pairs = (int64_t)d->batch * d->heads;
+  if (pairs <= 0 || pairs >= kXMinPairs) return 1;
+  const int64_t want = sm_count_of_current_device() / pairs;
+  return (int)std::max<int64_t>(1, std::min<int64_t>(want, xattn_key_tiles(d) / kXMinSplitTiles));
+}
+
+// fp32 partials: the forward's O_s, m_s, l_s; the backward's dQ_s (smaller) fits the same workspace
+size_t xattn_workspace_bytes(const svae_xattn_desc* d, int splits) {
+  if (splits <= 1) return 0;
+  return sizeof(float) * (size_t)d->batch * d->heads * splits * d->num_queries * (d->head_dim + 2);
+}
+
 template <typename T>
-static int launch_xattn_fwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v, const float* kpm, void* out,
-                            float* lse, cudaStream_t st) {
+static int launch_xattn_fwd(const svae_xattn_desc* d, int splits, const void* q, const void* k, const void* v, const float* kpm,
+                            void* out, float* lse, float* ws, cudaStream_t st) {
   constexpr int DH = 64;
   using S = XFwdSmem<DH>;
   CUtensorMap tmQ, tmK, tmV, tmO;
@@ -270,22 +359,36 @@ static int launch_xattn_fwd(const svae_xattn_desc* d, const void* q, const void*
   if ((rc = encode_tmap(&tmK, dt, k, DH, d->num_keys, d->heads, d->batch, d->k_stride, kTile))) return rc;
   if ((rc = encode_tmap(&tmV, dt, v, DH, d->num_keys, d->heads, d->batch, d->v_stride, kTile))) return rc;
   if ((rc = encode_tmap(&tmO, dt, out, DH, d->num_queries, d->heads, d->batch, d->o_stride, kTile))) return rc;
+  const int pairs = d->batch * d->heads;
+  const size_t parts = (size_t)pairs * splits * d->num_queries;
   XParams p;
   p.kpm = kpm; p.lse = lse; p.delta = nullptr;
+  p.part_o = splits > 1 ? ws : nullptr;
+  p.part_m = splits > 1 ? ws + parts * DH : nullptr;
+  p.part_l = splits > 1 ? ws + parts * (DH + 1) : nullptr;
   p.nq = d->num_queries; p.Lk = d->num_keys; p.H = d->heads;
   p.scale = d->scale; p.scale_log2 = d->scale * kLog2e;
   auto kern = xattn_fwd_sm100_kernel<T, DH>;
   SVAE_CONFIGURE_SMEM(kern, S::DYN_BYTES);
-  ScopedKernelTimer timer("xattn_fwd_sm100", st);
-  kern<<<d->batch * d->heads, kXThreads, S::DYN_BYTES, st>>>(tmQ, tmK, tmV, tmO, p);
-  SVAE_CUDA_CHECK(cudaGetLastError());
+  {
+    ScopedKernelTimer timer("xattn_fwd_sm100", st);
+    kern<<<dim3(pairs, splits), kXThreads, S::DYN_BYTES, st>>>(tmQ, tmK, tmV, tmO, p);
+    SVAE_CUDA_CHECK(cudaGetLastError());
+  }
+  if (splits > 1) {
+    ScopedKernelTimer timer("xattn_fwd_merge", st);
+    xattn_fwd_merge_kernel<T, DH><<<dim3(pairs, d->num_queries), DH, 0, st>>>(
+        p.part_o, p.part_m, p.part_l, reinterpret_cast<T*>(out), lse, d->o_stride[0], d->o_stride[1], d->o_stride[2], d->heads,
+        d->num_queries, splits);
+    SVAE_CUDA_CHECK(cudaGetLastError());
+  }
   return SVAE_OK;
 }
 
-int xattn_fwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v, const float* kpm, void* out, float* lse,
-              cudaStream_t st) {
-  return d->dtype == SVAE_DTYPE_BF16 ? launch_xattn_fwd<__nv_bfloat16>(d, q, k, v, kpm, out, lse, st)
-                                     : launch_xattn_fwd<__half>(d, q, k, v, kpm, out, lse, st);
+int xattn_fwd(const svae_xattn_desc* d, int splits, const void* q, const void* k, const void* v, const float* kpm, void* out,
+              float* lse, float* ws, cudaStream_t st) {
+  return d->dtype == SVAE_DTYPE_BF16 ? launch_xattn_fwd<__nv_bfloat16>(d, splits, q, k, v, kpm, out, lse, ws, st)
+                                     : launch_xattn_fwd<__half>(d, splits, q, k, v, kpm, out, lse, ws, st);
 }
 
 
@@ -312,6 +415,7 @@ struct XBwdParams {
   const float* lse;
   const void *out, *dout;       // read directly for delta = rowsum(dO o O)
   void* dq;
+  float* part_dq;               // key_splits > 1: [B*H][splits][nq][DH] the split's dQ_s, fp32
   int64_t o_stride[3], do_stride[3], dq_stride[3];
   int nq, Lk, H;
   float scale, scale_log2;
@@ -343,7 +447,9 @@ xattn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
 
   const int warp = warp_index(), lane = threadIdx.x & 31;
   const int h = blockIdx.x % p.H, b = blockIdx.x / p.H;
-  const int nt = (p.Lk + kTile - 1) / kTile;
+  int t0, t1;                                          // this CTA's key tiles (all of them with one split)
+  x_split_tiles((p.Lk + kTile - 1) / kTile, gridDim.y, blockIdx.y, t0, t1);
+  const int nt = t1 - t0;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kXStages; ++s) { mbar_init(k_full + s, 1); mbar_init(v_full + s, 1); mbar_init(kv_free + s, 1); }
@@ -405,9 +511,9 @@ xattn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
         const int s = i % kXStages;
         if (i >= kXStages) mbar_wait(kv_free + s, ((i / kXStages) - 1) & 1);
         mbar_arrive_expect_tx_w(k_full + s, S::TILE);
-        tma_load_4d_w(smem + S::OFF_K + s * S::TILE, &tmK, k_full + s, 0, i * kTile, h, b);
+        tma_load_4d_w(smem + S::OFF_K + s * S::TILE, &tmK, k_full + s, 0, (t0 + i) * kTile, h, b);
         mbar_arrive_expect_tx_w(v_full + s, S::TILE);
-        tma_load_4d_w(smem + S::OFF_V + s * S::TILE, &tmV, v_full + s, 0, i * kTile, h, b);
+        tma_load_4d_w(smem + S::OFF_V + s * S::TILE, &tmV, v_full + s, 0, (t0 + i) * kTile, h, b);
       }
     } else if (warp == 13) {
       // ---- S^T = K Q^T and dP^T = V dO^T (128 keys x 64 queries) into the score buffer of group i & 1
@@ -494,16 +600,33 @@ xattn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       fence_proxy_async();
       named_bar_sync(1, 128);
       if (tid_g == 0) {
-        tma_store_4d(&tmDK, stage[0], 0, i * kTile, h, b);       // rows beyond Lk are outside the tensor: clipped
-        tma_store_4d(&tmDV, stage[1], 0, i * kTile, h, b);
+        tma_store_4d(&tmDK, stage[0], 0, (t0 + i) * kTile, h, b);  // rows beyond Lk are outside the tensor: clipped
+        tma_store_4d(&tmDV, stage[1], 0, (t0 + i) * kTile, h, b);
         tma_store_commit();
         tma_store_wait_read();
         mbar_arrive(kv_free + s);
       }
     }
-    // dQ (complete after the last tile's MMAs): rows < nq, written directly.  tcgen05.ld is warp-collective: every lane
-    // of a warp that owns at least one query takes part in the loads, only the rows that exist are stored.
-    if (w * 32 < p.nq) {
+    // dQ (complete after the last tile's MMAs): rows < nq, written directly -- or, as one split of several, drained in
+    // fp32 for the reduce launch.  tcgen05.ld is warp-collective: every lane of a warp that owns at least one query takes
+    // part in the loads, only the rows that exist are stored.
+    if (gridDim.y > 1) {
+      if (w * 32 < p.nq) {
+        float* part = p.part_dq + (((int64_t)blockIdx.x * gridDim.y + blockIdx.y) * p.nq + row) * DH;
+#pragma unroll
+        for (int half = 0; half < DH / 32; ++half) {
+          uint32_t v[32];
+          tmem_ld32(trow + S::COL_DQ + 32 * half, v);
+          tmem_wait_ld(v);
+          if (row < p.nq) {
+#pragma unroll
+            for (int e = 0; e < 8; ++e)
+              reinterpret_cast<float4*>(part)[half * 8 + e] = make_float4(__uint_as_float(v[4 * e]), __uint_as_float(v[4 * e + 1]),
+                                                                           __uint_as_float(v[4 * e + 2]), __uint_as_float(v[4 * e + 3]));
+          }
+        }
+      }
+    } else if (w * 32 < p.nq) {
       T* dq = reinterpret_cast<T*>(p.dq) + b * p.dq_stride[0] + h * p.dq_stride[1] + row * p.dq_stride[2];
 #pragma unroll
       for (int half = 0; half < DH / 32; ++half) {
@@ -532,7 +655,7 @@ xattn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     const uint32_t trow = tmem_base + ((uint32_t)(c * 32) << 16);
     uint8_t* sDS = smem + S::OFF_DS;
     for (int i = wg; i < nt; i += 2) {
-      const int key = i * kTile + row;
+      const int key = (t0 + i) * kTile + row;
       float kv = -INFINITY;                              // additive key term (log2 domain); -inf beyond the sequence
       if (key < p.Lk) kv = p.kpm ? p.kpm[(int64_t)b * p.Lk + key] * kLog2e : 0.f;
       const uint32_t tb = trow + S::COL_U + 128 * wg;
@@ -589,9 +712,22 @@ xattn_bwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
   if (warp == 15) tmem_dealloc<512>(tmem_base);
 }
 
+// grid (B * H, nq), DH threads: dq = sum_s dQ_s over the splits in order, rounded once to 16 bits
+template <typename T, int DH>
+__global__ void __launch_bounds__(DH)
+xattn_dq_reduce_kernel(const float* __restrict__ part_dq, T* __restrict__ dq, int64_t s0, int64_t s1, int64_t s2, int H, int nq,
+                       int splits) {
+  const int pair = blockIdx.x, row = blockIdx.y, c = threadIdx.x, b = pair / H, h = pair - b * H;
+  const int64_t base = (int64_t)pair * splits;
+  float acc = 0.f;
+  for (int s = 0; s < splits; ++s) acc += part_dq[((base + s) * nq + row) * DH + c];
+  dq[b * s0 + h * s1 + row * s2 + c] = from_f32<T>(acc);
+}
+
 template <typename T>
-static int launch_xattn_bwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v, const void* out, const void* dout,
-                            const float* lse, const float* kpm, void* dq, void* dk, void* dv, cudaStream_t st) {
+static int launch_xattn_bwd(const svae_xattn_desc* d, int splits, const void* q, const void* k, const void* v, const void* out,
+                            const void* dout, const float* lse, const float* kpm, void* dq, void* dk, void* dv, float* ws,
+                            cudaStream_t st) {
   constexpr int DH = 64;
   using S = XBwdSmem<DH>;
   CUtensorMap tmQ, tmDO, tmK, tmV, tmDK, tmDV;
@@ -605,21 +741,31 @@ static int launch_xattn_bwd(const svae_xattn_desc* d, const void* q, const void*
   if ((rc = encode_tmap(&tmDV, dt, dv, DH, d->num_keys, d->heads, d->batch, d->dv_stride, kTile))) return rc;
   XBwdParams p;
   p.kpm = kpm; p.lse = lse; p.out = out; p.dout = dout; p.dq = dq;
+  p.part_dq = splits > 1 ? ws : nullptr;
   for (int i = 0; i < 3; ++i) { p.o_stride[i] = d->o_stride[i]; p.do_stride[i] = d->do_stride[i]; p.dq_stride[i] = d->dq_stride[i]; }
   p.nq = d->num_queries; p.Lk = d->num_keys; p.H = d->heads;
   p.scale = d->scale; p.scale_log2 = d->scale * kLog2e;
   auto kern = xattn_bwd_sm100_kernel<T, DH>;
   SVAE_CONFIGURE_SMEM(kern, S::DYN_BYTES);
-  ScopedKernelTimer timer("xattn_bwd_sm100", st);
-  kern<<<d->batch * d->heads, kXBThreads, S::DYN_BYTES, st>>>(tmQ, tmDO, tmK, tmV, tmDK, tmDV, p);
-  SVAE_CUDA_CHECK(cudaGetLastError());
+  const int pairs = d->batch * d->heads;
+  {
+    ScopedKernelTimer timer("xattn_bwd_sm100", st);
+    kern<<<dim3(pairs, splits), kXBThreads, S::DYN_BYTES, st>>>(tmQ, tmDO, tmK, tmV, tmDK, tmDV, p);
+    SVAE_CUDA_CHECK(cudaGetLastError());
+  }
+  if (splits > 1) {
+    ScopedKernelTimer timer("xattn_bwd_dq_reduce", st);
+    xattn_dq_reduce_kernel<T, DH><<<dim3(pairs, d->num_queries), DH, 0, st>>>(
+        ws, reinterpret_cast<T*>(dq), d->dq_stride[0], d->dq_stride[1], d->dq_stride[2], d->heads, d->num_queries, splits);
+    SVAE_CUDA_CHECK(cudaGetLastError());
+  }
   return SVAE_OK;
 }
 
-int xattn_bwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v, const void* out, const void* dout,
-              const float* lse, const float* kpm, void* dq, void* dk, void* dv, cudaStream_t st) {
-  return d->dtype == SVAE_DTYPE_BF16 ? launch_xattn_bwd<__nv_bfloat16>(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, st)
-                                     : launch_xattn_bwd<__half>(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, st);
+int xattn_bwd(const svae_xattn_desc* d, int splits, const void* q, const void* k, const void* v, const void* out, const void* dout,
+              const float* lse, const float* kpm, void* dq, void* dk, void* dv, float* ws, cudaStream_t st) {
+  return d->dtype == SVAE_DTYPE_BF16 ? launch_xattn_bwd<__nv_bfloat16>(d, splits, q, k, v, out, dout, lse, kpm, dq, dk, dv, ws, st)
+                                     : launch_xattn_bwd<__half>(d, splits, q, k, v, out, dout, lse, kpm, dq, dk, dv, ws, st);
 }
 
 }  // namespace sm100
@@ -633,25 +779,83 @@ static bool x_tma_ok(const void* p, const int64_t s[3]) {
 
 extern "C" int svae_xattn_supported(const svae_xattn_desc* d) { return d && sm100::xattn_supported(d) ? 1 : 0; }
 
-extern "C" int svae_xattn_fwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v,
-                              const float* key_padding_mask, void* out, float* lse, void* stream) {
-  SVAE_REQUIRE(d && q && k && v && out && lse, SVAE_ERR_INVALID, "svae_xattn_fwd: null argument");
+// the checks of the forward / backward entries; `name` is the entry that reports a failure
+static int x_check_fwd(const char* name, const svae_xattn_desc* d, const void* q, const void* k, const void* v, const void* out,
+                       const float* lse) {
+  SVAE_REQUIRE(d && q && k && v && out && lse, SVAE_ERR_INVALID, "%s: null argument", name);
   SVAE_REQUIRE(sm100::xattn_supported(d), SVAE_ERR_UNSUPPORTED,
-               "svae_xattn_fwd: needs 16-bit tensors, head_dim 64 and 1..128 queries (got dtype %d, head_dim %d, %d queries)", d->dtype,
+               "%s: needs 16-bit tensors, head_dim 64 and 1..128 queries (got dtype %d, head_dim %d, %d queries)", name, d->dtype,
                d->head_dim, d->num_queries);
   SVAE_REQUIRE(x_tma_ok(q, d->q_stride) && x_tma_ok(k, d->k_stride) && x_tma_ok(v, d->v_stride) && x_tma_ok(out, d->o_stride),
-               SVAE_ERR_INVALID, "svae_xattn_fwd: tensors must be 16-byte aligned with strides that are multiples of 8 elements");
-  return sm100::xattn_fwd(d, q, k, v, key_padding_mask, out, lse, static_cast<cudaStream_t>(stream));
+               SVAE_ERR_INVALID, "%s: tensors must be 16-byte aligned with strides that are multiples of 8 elements", name);
+  return SVAE_OK;
+}
+
+static int x_check_bwd(const char* name, const svae_xattn_desc* d, const void* q, const void* k, const void* v, const void* out,
+                       const void* dout, const float* lse, const void* dq, const void* dk, const void* dv) {
+  SVAE_REQUIRE(d && q && k && v && out && dout && lse && dq && dk && dv, SVAE_ERR_INVALID, "%s: null argument", name);
+  SVAE_REQUIRE(sm100::xattn_supported(d), SVAE_ERR_UNSUPPORTED, "%s: needs 16-bit tensors, head_dim 64 and 1..128 queries", name);
+  SVAE_REQUIRE(d->num_queries <= 64, SVAE_ERR_UNSUPPORTED, "%s: at most 64 queries (got %d)", name, d->num_queries);
+  SVAE_REQUIRE(x_tma_ok(q, d->q_stride) && x_tma_ok(k, d->k_stride) && x_tma_ok(v, d->v_stride) && x_tma_ok(out, d->o_stride) &&
+                   x_tma_ok(dout, d->do_stride) && x_tma_ok(dq, d->dq_stride) && x_tma_ok(dk, d->dk_stride) && x_tma_ok(dv, d->dv_stride),
+               SVAE_ERR_INVALID, "%s: tensors must be 16-byte aligned with strides that are multiples of 8 elements", name);
+  return SVAE_OK;
+}
+
+// key_splits within 1..key tiles and a workspace of svae_xattn_workspace_bytes (none needed for one split)
+static int x_check_split(const char* name, const svae_xattn_desc* d, int key_splits, const void* ws, size_t ws_bytes) {
+  const int tiles = sm100::xattn_key_tiles(d);
+  SVAE_REQUIRE(key_splits >= 1 && key_splits <= tiles, SVAE_ERR_INVALID, "%s: key_splits %d outside 1..%d (the 128-key tiles of %d keys)",
+               name, key_splits, tiles, d->num_keys);
+  const size_t need = sm100::xattn_workspace_bytes(d, key_splits);
+  SVAE_REQUIRE(need == 0 || (ws && ws_bytes >= need), SVAE_ERR_INVALID, "%s: workspace of %zu bytes at %p, %zu needed for %d key splits",
+               name, ws_bytes, ws, need, key_splits);
+  SVAE_REQUIRE(reinterpret_cast<uintptr_t>(ws) % 16 == 0, SVAE_ERR_INVALID, "%s: workspace must be 16-byte aligned", name);
+  return SVAE_OK;
+}
+
+extern "C" int svae_xattn_key_splits(const svae_xattn_desc* d) {
+  SVAE_REQUIRE(d && sm100::xattn_supported(d) && d->batch > 0 && d->heads > 0, SVAE_ERR_INVALID,
+               "svae_xattn_key_splits: null or unsupported descriptor");
+  return sm100::xattn_key_splits(d);
+}
+
+extern "C" size_t svae_xattn_workspace_bytes(const svae_xattn_desc* d, int key_splits) {
+  if (!d || !sm100::xattn_supported(d) || key_splits < 1 || key_splits > sm100::xattn_key_tiles(d)) return 0;
+  return sm100::xattn_workspace_bytes(d, key_splits);
+}
+
+extern "C" int svae_xattn_fwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v,
+                              const float* key_padding_mask, void* out, float* lse, void* stream) {
+  int rc;
+  if ((rc = x_check_fwd("svae_xattn_fwd", d, q, k, v, out, lse))) return rc;
+  return sm100::xattn_fwd(d, 1, q, k, v, key_padding_mask, out, lse, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int svae_xattn_fwd_split(const svae_xattn_desc* d, int key_splits, const void* q, const void* k, const void* v,
+                                    const float* key_padding_mask, void* out, float* lse, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
+  int rc;
+  if ((rc = x_check_fwd("svae_xattn_fwd_split", d, q, k, v, out, lse))) return rc;
+  if ((rc = x_check_split("svae_xattn_fwd_split", d, key_splits, workspace, workspace_bytes))) return rc;
+  return sm100::xattn_fwd(d, key_splits, q, k, v, key_padding_mask, out, lse, static_cast<float*>(workspace),
+                          static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int svae_xattn_bwd(const svae_xattn_desc* d, const void* q, const void* k, const void* v, const void* out,
                               const void* dout, const float* lse, const float* key_padding_mask, void* dq, void* dk, void* dv,
                               void* stream) {
-  SVAE_REQUIRE(d && q && k && v && out && dout && lse && dq && dk && dv, SVAE_ERR_INVALID, "svae_xattn_bwd: null argument");
-  SVAE_REQUIRE(sm100::xattn_supported(d), SVAE_ERR_UNSUPPORTED, "svae_xattn_bwd: needs 16-bit tensors, head_dim 64 and 1..128 queries");
-  SVAE_REQUIRE(d->num_queries <= 64, SVAE_ERR_UNSUPPORTED, "svae_xattn_bwd: at most 64 queries (got %d)", d->num_queries);
-  SVAE_REQUIRE(x_tma_ok(q, d->q_stride) && x_tma_ok(k, d->k_stride) && x_tma_ok(v, d->v_stride) && x_tma_ok(out, d->o_stride) &&
-                   x_tma_ok(dout, d->do_stride) && x_tma_ok(dq, d->dq_stride) && x_tma_ok(dk, d->dk_stride) && x_tma_ok(dv, d->dv_stride),
-               SVAE_ERR_INVALID, "svae_xattn_bwd: tensors must be 16-byte aligned with strides that are multiples of 8 elements");
-  return sm100::xattn_bwd(d, q, k, v, out, dout, lse, key_padding_mask, dq, dk, dv, static_cast<cudaStream_t>(stream));
+  int rc;
+  if ((rc = x_check_bwd("svae_xattn_bwd", d, q, k, v, out, dout, lse, dq, dk, dv))) return rc;
+  return sm100::xattn_bwd(d, 1, q, k, v, out, dout, lse, key_padding_mask, dq, dk, dv, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int svae_xattn_bwd_split(const svae_xattn_desc* d, int key_splits, const void* q, const void* k, const void* v,
+                                    const void* out, const void* dout, const float* lse, const float* key_padding_mask, void* dq,
+                                    void* dk, void* dv, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = x_check_bwd("svae_xattn_bwd_split", d, q, k, v, out, dout, lse, dq, dk, dv))) return rc;
+  if ((rc = x_check_split("svae_xattn_bwd_split", d, key_splits, workspace, workspace_bytes))) return rc;
+  return sm100::xattn_bwd(d, key_splits, q, k, v, out, dout, lse, key_padding_mask, dq, dk, dv, static_cast<float*>(workspace),
+                          static_cast<cudaStream_t>(stream));
 }
