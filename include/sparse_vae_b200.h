@@ -102,12 +102,15 @@ SVAE_API int svae_layout_build(int32_t num_blocks, int32_t window_size, int32_t 
 SVAE_API int svae_attn_fwd(const svae_attn_desc* desc, const void* q, const void* k, const void* v,
                   const float* key_padding_mask, void* out, float* lse, void* stream);
 
-/* Which kernels svae_attn_bwd will run for this problem: the tcgen05 kernels need 16-bit tensors, head_dim 64 and
- * a band of <= 13 key blocks; everything else takes the exact CUDA-core kernels (20-40x slower; the host wrapper
- * warns when 16-bit tensors end up there).  < 0: invalid descriptor. */
+/* Which kernels svae_attn_bwd will run for this problem: the tcgen05 kernels need 16-bit tensors and either head_dim
+ * 64 with a band of <= 13 key blocks or head_dim 128 with a causal layout and window 1..10; everything else takes the
+ * exact CUDA-core kernels (20-40x slower; the host wrapper warns when 16-bit tensors end up there), except 16-bit
+ * head_dim 128 outside its kernels (non-causal layouts, windows > 10), which is SVAE_ERR_UNSUPPORTED in both
+ * directions.  < 0: invalid descriptor or SVAE_ERR_UNSUPPORTED. */
 #define SVAE_BWD_PATH_TCGEN05 0            /* one pass over the sequence (causal, window <= 4: the reference's default) */
 #define SVAE_BWD_PATH_EXACT   1
 #define SVAE_BWD_PATH_TCGEN05_TWO_PASS 2   /* dQ pass + dK/dV pass (non-causal layouts, windows 5..10) */
+#define SVAE_BWD_PATH_TCGEN05_D128 3       /* head_dim 128, causal, windows 1..10: dQ pass + dK/dV pass, streamed slot groups */
 SVAE_API int svae_attn_bwd_path(const svae_attn_desc* desc);
 
 SVAE_API size_t svae_attn_bwd_workspace_bytes(const svae_attn_desc* desc);

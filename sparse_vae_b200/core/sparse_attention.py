@@ -97,7 +97,8 @@ class _SparseAttentionFn(torch.autograd.Function):
                 N.lib.svae_attn_bwd_path(ctypes.byref(desc)) == 1 and (Dh, cfg.window_size) not in _WARNED_EXACT:
             _WARNED_EXACT.add((Dh, cfg.window_size))
             warnings.warn(f"sparse attention backward: {q.dtype} tensors with head_dim {Dh} / window {cfg.window_size} are "
-                          f"outside the tensor-core kernels (head_dim 64, band <= 13 blocks) and run the exact CUDA-core "
+                          f"outside the tensor-core kernels (head_dim 64 with a band <= 13 blocks, head_dim 128 causal with "
+                          f"window 1..10) and run the exact CUDA-core "
                           f"kernels, 20-40x slower", RuntimeWarning, stacklevel=2)
         ws_bytes = N.lib.svae_attn_bwd_workspace_bytes(ctypes.byref(desc))
         ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=q.device)

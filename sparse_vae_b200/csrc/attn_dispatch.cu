@@ -1,6 +1,6 @@
 // C-ABI entry points of the attention path: argument validation, TMA descriptor encoding, path selection.
 //   fp32 tensors (or SVAE_ATTN_FORCE_EXACT)  -> exact CUDA-core kernels (attn_exact.cu)   [parity mode]
-//   bf16 / fp16 tensors                      -> tcgen05 / TMEM / TMA kernels (attn_*_sm100.cu)
+//   bf16 / fp16 tensors                      -> tcgen05 / TMEM / TMA kernels (attn_*_sm100.cu; head 128: attn_d128_sm100.cu)
 #include <mutex>
 
 #include "attn_sm100.cuh"
@@ -25,6 +25,11 @@ int bwd1(const svae_attn_desc*, const void*, const void*, const void*, const voi
          const float*, void*, void*, void*, void*, cudaStream_t);
 int bwd(const svae_attn_desc*, const void*, const void*, const void*, const void*, const void*, const float*,
         const float*, void*, void*, void*, void*, cudaStream_t);
+bool d128_supported(const svae_attn_desc*);
+size_t d128_bwd_workspace(const svae_attn_desc*);
+int d128_fwd(const svae_attn_desc*, const void*, const void*, const void*, const float*, void*, float*, cudaStream_t);
+int d128_bwd(const svae_attn_desc*, const void*, const void*, const void*, const void*, const void*, const float*,
+             const float*, void*, void*, void*, void*, cudaStream_t);
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -44,7 +49,8 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// 4-D map {Dh, L, H, B} over a strided [B, H, L, Dh] tensor; box = {Dh, box_rows, 1, 1}; swizzle = row bytes.
+// 4-D map {Dh, L, H, B} over a strided [B, H, L, Dh] tensor; box = {min(Dh, 64), box_rows, 1, 1}; swizzle = box row
+// bytes.  Rows wider than one 128-byte swizzle atom (Dh 128) arrive as several boxes of 64 columns.
 int encode_tmap(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int Dh, int L, int H, int B,
                 const int64_t stride[3], int box_rows) {
   // A tensor map is a pure function of (base, dtype, dims, strides, box): a training step asks for the same handful
@@ -78,9 +84,10 @@ int encode_tmap(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int 
   int64_t s_row = stride[2], s_head = H > 1 ? stride[1] : (int64_t)Dh, s_batch = B > 1 ? stride[0] : (int64_t)L * stride[2];
   if (L == 1) s_row = Dh;
   cuuint64_t strides[3] = {(cuuint64_t)(s_row * es), (cuuint64_t)(s_head * es), (cuuint64_t)(s_batch * es)};
-  cuuint32_t box[4] = {(cuuint32_t)Dh, (cuuint32_t)box_rows, 1, 1};
+  const int box_cols = Dh < 64 ? Dh : 64;
+  cuuint32_t box[4] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 1, 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  const int rowb = Dh * 2;
+  const int rowb = box_cols * 2;
   CUtensorMapSwizzle sw = rowb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : rowb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
                                                                                : CU_TENSOR_MAP_SWIZZLE_32B;
   CUresult r = fn(map, dt, 4, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
@@ -143,6 +150,10 @@ static bool use_exact(const svae_attn_desc* d) {
   return d->dtype == SVAE_DTYPE_F32 || (d->flags & SVAE_ATTN_FORCE_EXACT);
 }
 
+// 16-bit head 128: one kernel per direction (attn_d128_sm100.cu) for causal windows 1..10, otherwise unsupported;
+// SVAE_ATTN_PERSISTENT and SVAE_ATTN_BWD_TWO_PASS do not apply
+static bool use_d128(const svae_attn_desc* d) { return !use_exact(d) && d->head_dim == 128; }
+
 // one pass over the sequence (attn_bwd1_sm100.cu) unless the geometry is outside it or the caller asks for the
 // two-pass kernels (attn_bwd_sm100.cu: non-causal layouts and windows 5..10)
 static bool use_one_pass(const svae_attn_desc* d) {
@@ -168,9 +179,11 @@ static int attn_fwd_impl(const svae_attn_desc* d, const void* q, const void* k, 
     SVAE_REQUIRE(s_dump == nullptr, SVAE_ERR_UNSUPPORTED, "score dump is only implemented on the sm100 path");
     return exact_fwd(d, q, k, v, kpm, out, lse, st);
   }
+  SVAE_REQUIRE(!(use_d128(d) && s_dump), SVAE_ERR_UNSUPPORTED, "score dump is not implemented at head_dim 128");
   SVAE_REQUIRE(tma_ok(q, d->q_stride, d->heads, d->batch, d->seq_len) && tma_ok(k, d->k_stride, d->heads, d->batch, d->seq_len) &&
                    tma_ok(v, d->v_stride, d->heads, d->batch, d->seq_len) && tma_ok(out, d->o_stride, d->heads, d->batch, d->seq_len),
                SVAE_ERR_INVALID, "svae_attn_fwd: 16-bit tensors must be 16-byte aligned with strides that are multiples of 8 elements");
+  if (use_d128(d)) return sm100::d128_fwd(d, q, k, v, kpm, out, lse, st);
   // persistent warp-specialised kernel (69 us vs 104 us at the C2 shape): what the host wrapper asks for whenever the
   // geometry fits (<= 8 key slots); wider windows and score dumps take the one-CTA-per-tile kernel
   if (!s_dump && (d->flags & SVAE_ATTN_PERSISTENT) && sm100::fwd_persist_supported(d))
@@ -192,6 +205,7 @@ extern "C" int svae_attn_fwd_debug(const svae_attn_desc* d, const void* q, const
 
 extern "C" size_t svae_attn_bwd_workspace_bytes(const svae_attn_desc* d) {
   if (validate(d, true)) return 0;
+  if (use_d128(d)) return sm100::d128_supported(d) ? sm100::d128_bwd_workspace(d) : 0;
   if (use_exact(d) || !sm100::bwd_supported(d)) return exact_bwd_workspace(d);
   if (use_one_pass(d)) return sm100::bwd1_workspace(d);
   return sm100::bwd_workspace(d);
@@ -199,6 +213,7 @@ extern "C" size_t svae_attn_bwd_workspace_bytes(const svae_attn_desc* d) {
 
 extern "C" int svae_attn_bwd_path(const svae_attn_desc* d) {
   if (validate(d, true)) return -1;
+  if (use_d128(d)) return sm100::d128_supported(d) ? SVAE_BWD_PATH_TCGEN05_D128 : SVAE_ERR_UNSUPPORTED;
   if (use_exact(d) || !sm100::bwd_supported(d)) return SVAE_BWD_PATH_EXACT;
   return use_one_pass(d) ? SVAE_BWD_PATH_TCGEN05 : SVAE_BWD_PATH_TCGEN05_TWO_PASS;
 }
@@ -215,12 +230,13 @@ extern "C" int svae_attn_bwd(const svae_attn_desc* d, const void* q, const void*
                svae_attn_bwd_workspace_bytes(d));
   SVAE_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 256 == 0, SVAE_ERR_INVALID, "svae_attn_bwd: workspace must be 256-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (use_exact(d) || !sm100::bwd_supported(d)) return exact_bwd(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, workspace, st);
+  if (!use_d128(d) && (use_exact(d) || !sm100::bwd_supported(d))) return exact_bwd(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, workspace, st);
   const bool ok = tma_ok(q, d->q_stride, d->heads, d->batch, d->seq_len) && tma_ok(k, d->k_stride, d->heads, d->batch, d->seq_len) &&
                   tma_ok(v, d->v_stride, d->heads, d->batch, d->seq_len) && tma_ok(out, d->o_stride, d->heads, d->batch, d->seq_len) &&
                   tma_ok(dout, d->do_stride, d->heads, d->batch, d->seq_len) && tma_ok(dq, d->dq_stride, d->heads, d->batch, d->seq_len) &&
                   tma_ok(dk, d->dk_stride, d->heads, d->batch, d->seq_len) && tma_ok(dv, d->dv_stride, d->heads, d->batch, d->seq_len);
   SVAE_REQUIRE(ok, SVAE_ERR_INVALID, "svae_attn_bwd: 16-bit tensors must be 16-byte aligned with strides that are multiples of 8 elements");
+  if (use_d128(d)) return sm100::d128_bwd(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, workspace, st);
   if (use_one_pass(d)) return sm100::bwd1(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, workspace, st);
   return sm100::bwd(d, q, k, v, out, dout, lse, kpm, dq, dk, dv, workspace, st);
 }

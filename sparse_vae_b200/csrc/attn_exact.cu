@@ -64,7 +64,15 @@ constexpr int kMaxLive = 64;
 template <typename T, int DH>
 __global__ void __launch_bounds__(kExThreads) attn_exact_fwd_kernel(ExactArgs a) {
   constexpr int LD = DH + 1;
-  __shared__ float Qs[kBlk * LD], Ks[kBlk * LD], Vs[kBlk * LD], Ps[kBlk * (kBlk + 1)];
+  // head 128: the tiles exceed 48 KB of static shared memory and live in the dynamic allocation instead
+  constexpr bool kDyn = DH > 64;
+  __shared__ float Qs_[kDyn ? 1 : kBlk * LD], Ks_[kDyn ? 1 : kBlk * LD], Vs_[kDyn ? 1 : kBlk * LD],
+      Ps_[kDyn ? 1 : kBlk * (kBlk + 1)];
+  extern __shared__ float dyn_tiles[];
+  float* Qs = kDyn ? dyn_tiles : Qs_;
+  float* Ks = kDyn ? dyn_tiles + kBlk * LD : Ks_;
+  float* Vs = kDyn ? dyn_tiles + 2 * kBlk * LD : Vs_;
+  float* Ps = kDyn ? dyn_tiles + 3 * kBlk * LD : Ps_;
   __shared__ float kpm_s[kBlk];
   __shared__ int live[kMaxLive];
   __shared__ int nlive;
@@ -147,8 +155,17 @@ __global__ void __launch_bounds__(kExThreads) attn_exact_fwd_kernel(ExactArgs a)
 template <typename T, int DH>
 __global__ void __launch_bounds__(kExThreads) attn_exact_bwd_kernel(ExactArgs a) {
   constexpr int LD = DH + 1;
-  __shared__ float Qs[kBlk * LD], Ks[kBlk * LD], Vs[kBlk * LD], dOs[kBlk * LD];
-  __shared__ float Ps[kBlk * (kBlk + 1)], dSs[kBlk * (kBlk + 1)];
+  constexpr bool kDyn = DH > 64;                      // see attn_exact_fwd_kernel
+  __shared__ float Qs_[kDyn ? 1 : kBlk * LD], Ks_[kDyn ? 1 : kBlk * LD], Vs_[kDyn ? 1 : kBlk * LD],
+      dOs_[kDyn ? 1 : kBlk * LD];
+  __shared__ float Ps_[kDyn ? 1 : kBlk * (kBlk + 1)], dSs_[kDyn ? 1 : kBlk * (kBlk + 1)];
+  extern __shared__ float dyn_tiles[];
+  float* Qs = kDyn ? dyn_tiles : Qs_;
+  float* Ks = kDyn ? dyn_tiles + kBlk * LD : Ks_;
+  float* Vs = kDyn ? dyn_tiles + 2 * kBlk * LD : Vs_;
+  float* dOs = kDyn ? dyn_tiles + 3 * kBlk * LD : dOs_;
+  float* Ps = kDyn ? dyn_tiles + 4 * kBlk * LD : Ps_;
+  float* dSs = kDyn ? dyn_tiles + 4 * kBlk * LD + kBlk * (kBlk + 1) : dSs_;
   __shared__ float kpm_s[kBlk];
   __shared__ int live[kMaxLive];
   __shared__ int nlive;
@@ -285,7 +302,14 @@ static int launch_fwd_t(const ExactArgs& a, cudaStream_t st) {
     case 16: attn_exact_fwd_kernel<T, 16><<<grid, kExThreads, 0, st>>>(a); break;
     case 32: attn_exact_fwd_kernel<T, 32><<<grid, kExThreads, 0, st>>>(a); break;
     case 64: attn_exact_fwd_kernel<T, 64><<<grid, kExThreads, 0, st>>>(a); break;
-    default: SVAE_REQUIRE(false, SVAE_ERR_UNSUPPORTED, "exact attention: head_dim %d not in {16,32,64}", a.Dh);
+    case 128: {
+      constexpr int bytes = (3 * kBlk * 129 + kBlk * (kBlk + 1)) * 4;
+      auto kern = attn_exact_fwd_kernel<T, 128>;
+      SVAE_CONFIGURE_SMEM(kern, bytes);
+      kern<<<grid, kExThreads, bytes, st>>>(a);
+      break;
+    }
+    default: SVAE_REQUIRE(false, SVAE_ERR_UNSUPPORTED, "exact attention: head_dim %d not in {16,32,64,128}", a.Dh);
   }
   SVAE_CUDA_CHECK(cudaGetLastError());
   return SVAE_OK;
@@ -301,7 +325,14 @@ static int launch_bwd_t(const ExactArgs& a, const svae_attn_desc* d, void* dk, v
     case 16: attn_exact_bwd_kernel<T, 16><<<grid, kExThreads, 0, st>>>(a); break;
     case 32: attn_exact_bwd_kernel<T, 32><<<grid, kExThreads, 0, st>>>(a); break;
     case 64: attn_exact_bwd_kernel<T, 64><<<grid, kExThreads, 0, st>>>(a); break;
-    default: SVAE_REQUIRE(false, SVAE_ERR_UNSUPPORTED, "exact attention: head_dim %d not in {16,32,64}", a.Dh);
+    case 128: {
+      constexpr int bytes = (4 * kBlk * 129 + 2 * kBlk * (kBlk + 1)) * 4;
+      auto kern = attn_exact_bwd_kernel<T, 128>;
+      SVAE_CONFIGURE_SMEM(kern, bytes);
+      kern<<<grid, kExThreads, bytes, st>>>(a);
+      break;
+    }
+    default: SVAE_REQUIRE(false, SVAE_ERR_UNSUPPORTED, "exact attention: head_dim %d not in {16,32,64,128}", a.Dh);
   }
   SVAE_CUDA_CHECK(cudaGetLastError());
   int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);

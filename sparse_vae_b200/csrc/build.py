@@ -18,7 +18,7 @@ ROOT = HERE.parents[1]
 BUILD = HERE / 'build'
 LIB = HERE / 'libsvae_b200.so'
 SOURCES = ['abi.cu', 'bottleneck.cu', 'attn_exact.cu', 'attn_fwd_sm100.cu', 'attn_fwd_persist_sm100.cu', 'attn_bwd_sm100.cu',
-           'attn_bwd1_sm100.cu', 'xattn_sm100.cu', 'causal_attn_sm100.cu', 'attn_dispatch.cu', 'optim.cu', 'layernorm.cu', 'vocab_ce.cu', 'rotary.cu', 'colsum.cu',
+           'attn_bwd1_sm100.cu', 'attn_d128_sm100.cu', 'xattn_sm100.cu', 'causal_attn_sm100.cu', 'attn_dispatch.cu', 'optim.cu', 'layernorm.cu', 'vocab_ce.cu', 'rotary.cu', 'colsum.cu',
            'decode_attn.cu', 'decode_attn_dense.cu', 'sampling.cu', 'residual.cu', 'gelu.cu', 'embedding.cu', 'vocab_ll_sm100.cu']
 HEADERS = ['common.cuh', 'sm100_ptx.cuh', 'attn_sm100.cuh', '../../include/sparse_vae_b200.h']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',

@@ -46,7 +46,7 @@ __global__ void __launch_bounds__(480) decode_attn_kernel(const T* __restrict__ 
                                                            int block, int table_rows, int64_t in_stride, float scale) {
   constexpr int kVec = 16 / sizeof(T);              // elements per 16-byte load
   constexpr int kMaxWarps = 15;                     // window <= 14
-  constexpr int kPer = DH / 32;                     // output features per lane (1 or 2)
+  constexpr int kPer = DH / 32;                     // output features per lane (1, 2 or 4)
   __shared__ float s_q[HPC][DH];
   __shared__ float s_max[HPC][kMaxWarps], s_sum[HPC][kMaxWarps];
   __shared__ float s_out[HPC][kMaxWarps][DH];
@@ -65,10 +65,10 @@ __global__ void __launch_bounds__(480) decode_attn_kernel(const T* __restrict__ 
   const size_t out_row = (size_t)b * d_model + (size_t)h0 * DH;
   T* kc = key_cache + ((size_t)b * C) * d_model + (size_t)h0 * DH;
   T* vc = value_cache + ((size_t)b * C) * d_model + (size_t)h0 * DH;
-  if (warp == 0 && lane < DH / 2) {
+  for (int pr = lane; warp == 0 && pr < DH / 2; pr += 32) {     // rotary pair pr (head 128: two per lane)
 #pragma unroll
     for (int hh = 0; hh < HPC; ++hh) {
-      const int f = hh * DH + 2 * lane;             // feature offset inside this CTA's head group
+      const int f = hh * DH + 2 * pr;               // feature offset inside this CTA's head group
       const float c = cos_t[(size_t)trow * (d_model / 2) + (h0 * DH + f) / 2];
       const float s = sin_t[(size_t)trow * (d_model / 2) + (h0 * DH + f) / 2];
       const float qe = to_f32<T>(q[row + f]), qo = to_f32<T>(q[row + f + 1]);
@@ -77,8 +77,8 @@ __global__ void __launch_bounds__(480) decode_attn_kernel(const T* __restrict__ 
       const T q1 = from_f32<T>(__fadd_rn(__fmul_rn(qo, c), __fmul_rn(qe, s)));
       const T k0 = from_f32<T>(__fsub_rn(__fmul_rn(ke, c), __fmul_rn(ko, s)));
       const T k1 = from_f32<T>(__fadd_rn(__fmul_rn(ko, c), __fmul_rn(ke, s)));
-      s_q[hh][2 * lane] = to_f32<T>(q0);
-      s_q[hh][2 * lane + 1] = to_f32<T>(q1);
+      s_q[hh][2 * pr] = to_f32<T>(q0);
+      s_q[hh][2 * pr + 1] = to_f32<T>(q1);
       kc[(size_t)slot * d_model + f] = k0;
       kc[(size_t)slot * d_model + f + 1] = k1;
       vc[(size_t)slot * d_model + f] = v[row + f];
@@ -176,7 +176,7 @@ static int launch_decode(const void* q, const void* k, const void* v, const floa
       (const T*)q, (const T*)k, (const T*)v, c, s, (T*)kc, (T*)vc, (T*)out, pos, B, H, window, block, table_rows, in_stride, scale)
   // HPC = 2 (half the CTAs, twice the loads in flight per lane) measured slower on B200: 29 us vs 21 us per launch at
   // 256 samples x 8 heads x 160 slots -- its registers cost more residency than the extra loads buy
-  if (Dh == 64) SVAE_DEC(64, 1); else SVAE_DEC(32, 1);
+  if (Dh == 128) SVAE_DEC(128, 1); else if (Dh == 64) SVAE_DEC(64, 1); else SVAE_DEC(32, 1);
 #undef SVAE_DEC
   SVAE_CUDA_CHECK(cudaGetLastError());
   return SVAE_OK;
@@ -187,7 +187,7 @@ static int launch_decode(const void* q, const void* k, const void* v, const floa
 using namespace svae;
 
 extern "C" int svae_decode_attn_supported(int32_t head_dim, int32_t window, int32_t block) {
-  return (head_dim == 32 || head_dim == 64) && window >= 1 && window <= 14 && block == 32;
+  return (head_dim == 32 || head_dim == 64 || head_dim == 128) && window >= 1 && window <= 14 && block == 32;
 }
 
 extern "C" int svae_decode_attn(const void* q, const void* k, const void* v, const float* cos_table,
@@ -199,7 +199,7 @@ extern "C" int svae_decode_attn(const void* q, const void* k, const void* v, con
   SVAE_REQUIRE(q && k && v && cos_table && sin_table && key_cache && value_cache && out && position, SVAE_ERR_INVALID,
                "svae_decode_attn: null argument");
   SVAE_REQUIRE(svae_decode_attn_supported(head_dim, window, block), SVAE_ERR_UNSUPPORTED,
-               "svae_decode_attn: head_dim %d / window %d / block %d not supported (head_dim 32|64, window 1..14, block 32)",
+               "svae_decode_attn: head_dim %d / window %d / block %d not supported (head_dim 32|64|128, window 1..14, block 32)",
                head_dim, window, block);
   SVAE_REQUIRE(B >= 0 && H > 0 && table_rows > 0 && in_stride >= (int64_t)H * head_dim && in_stride % 8 == 0,
                SVAE_ERR_INVALID, "svae_decode_attn: bad sizes");
