@@ -222,9 +222,9 @@ SVAE_API int svae_xattn_bwd_split(const svae_xattn_desc* desc, int key_splits, c
 /* ---- dense CAUSAL self-attention with additive key padding (the non-sparse decoders in training; reference
  * core/attention.py:83-100 with causal=True and a padding mask).  Uses svae_xattn_desc with num_queries == num_keys = L:
  *   out[b,h,i,:] = softmax_{j <= i}(scale * q_i . k_j + key_padding_mask[b, j]) v_j ; lse: fp32 [batch, heads, L], natural log.
- * Keys j > i never enter the sum.  key_padding_mask: additive fp32 [batch, L] or NULL.  16-bit, head_dim 64, any L >= 1;
- * q/k/v/out/dout/dq/dk/dv 16-byte aligned with strides that are multiples of 8 elements.  Deterministic (no atomics),
- * no host synchronisation. */
+ * Keys j > i never enter the sum.  key_padding_mask: additive fp32 [batch, L] or NULL.  16-bit, head_dim 64 or 128,
+ * any L >= 1; q/k/v/out/dout/dq/dk/dv 16-byte aligned with strides that are multiples of 8 elements.  Deterministic
+ * (no atomics), no host synchronisation. */
 SVAE_API int svae_causal_attn_supported(const svae_xattn_desc* desc);
 SVAE_API int svae_causal_attn_fwd(const svae_xattn_desc* desc, const void* q, const void* k, const void* v,
                          const float* key_padding_mask, void* out, float* lse, void* stream);
@@ -383,7 +383,7 @@ SVAE_API int svae_decode_attn(const void* q, const void* k, const void* v, const
  *                         (may be null when that is 0); holds the per-split partial results.
  * Split-KV: the live slots are dealt out to a number of CTAs per (sample, head) fixed by B, H and cache_len, and their
  * partial softmax results are merged in a fixed order (no atomics): bit-identical from run to run, graph-capturable.
- * position >= cache_len reads and writes nothing.  head_dim 32 | 64, cache_len 1..65536. */
+ * position >= cache_len reads and writes nothing.  head_dim 32 | 64 | 128, cache_len 1..65536. */
 SVAE_API int svae_decode_attn_dense_supported(int32_t head_dim, int32_t cache_len);
 SVAE_API size_t svae_decode_attn_dense_workspace_bytes(int32_t B, int32_t H, int32_t head_dim, int32_t cache_len);
 SVAE_API int svae_decode_attn_dense(const void* q, const void* k, const void* v, const float* cos_table,

@@ -86,19 +86,19 @@ class _CausalAttentionFn(torch.autograd.Function):
 
 
 def supported(q: Tensor, k: Tensor, v: Tensor) -> bool:
-    """CUDA tensors [B, H, L, 64] of one 16-bit dtype, q / k / v of one shape, unit inner stride."""
+    """CUDA tensors [B, H, L, 64] or [B, H, L, 128] of one 16-bit dtype, q / k / v of one shape, unit inner stride."""
     return (q.is_cuda and q.ndim == 4 and q.dtype in (torch.bfloat16, torch.float16) and q.dtype == k.dtype == v.dtype
-            and q.shape[-1] == 64 and q.shape == k.shape == v.shape and q.shape[-2] >= 1
+            and q.shape[-1] in (64, 128) and q.shape == k.shape == v.shape and q.shape[-2] >= 1
             and q.stride(-1) == 1 and k.stride(-1) == 1 and v.stride(-1) == 1)
 
 
 def causal_attention(q: Tensor, k: Tensor, v: Tensor, key_padding_mask: Tensor = None, joint_grads: bool = False) -> Tensor:
-    """softmax_{j <= i}(q_i k_j^T / sqrt(d) + key_padding_mask[:, None, j]) v for q / k / v [B, H, L, 64];
+    """softmax_{j <= i}(q_i k_j^T / sqrt(d) + key_padding_mask[:, None, j]) v for q / k / v [B, H, L, Dh], Dh 64 or 128;
     `key_padding_mask` additive fp32 [B, L] (or [1, L]) or None.  Returns [B, H, L, Dh] as a view of [B, L, H, Dh]
     memory.  `joint_grads`: the backward writes dq | dk | dv into one [B, L, 3, H, Dh] buffer."""
     _bind()
     if not supported(q, k, v):
-        raise ValueError(f"causal_attention needs CUDA tensors [B, H, L, 64] of one 16-bit dtype with unit inner stride; got "
+        raise ValueError(f"causal_attention needs CUDA tensors [B, H, L, 64 or 128] of one 16-bit dtype with unit inner stride; got "
                          f"{q.dtype} {tuple(q.shape)}, {k.dtype} {tuple(k.shape)}, {v.dtype} {tuple(v.shape)}")
     kpm = None
     if key_padding_mask is not None:

@@ -64,8 +64,8 @@ def attention_kind(layer, cache_len: int) -> Optional[str]:
 
 def supported(model, state: GenerationState) -> bool:
     """Graphed decoding covers CUDA models whose every decoder layer is causal self-attention without cross-attention,
-    either block-sparse (global first block, head size 32, 64 or 128) or dense (head size 32 or 64).  Anything else keeps the module-by-module
-    sampler."""
+    either block-sparse (global first block, head size 32, 64 or 128) or dense (head size 32, 64 or 128).  Anything else
+    keeps the module-by-module sampler."""
     if not (N.FUSED_EXTRAS and model.device.type == 'cuda' and len(model.decoder_layers) > 0):
         return False
     if len(model.input_layer) != 2 or state.output_ids.dtype != torch.long:

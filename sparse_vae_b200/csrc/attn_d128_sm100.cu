@@ -7,9 +7,8 @@
 // causal_attn_sm100.cu: 6 warps, warps 0-3 math (one TMEM lane quarter = one 32-row block each, so block sparsity is
 // warp-uniform), warp 4 TMA, warp 5 MMA issue.
 //
-// Operand layout: a 128-element row is 256 bytes = two SWIZZLE_128B atoms, so every 128-row operand tile arrives as two
-// TMA boxes of 64 columns, stored as two 16 KB halves.  K-major operands (Q K^T) step through both halves; MN-major
-// operands (P V, dS K, P^T dO) span them with the descriptor's leading-byte offset = 16 KB.
+// Operand layout (attn_sm100.cuh, kmajor_desc / mnmajor_desc): every 128-row operand tile arrives as two TMA boxes of
+// 64 columns, stored as two 16 KB halves.
 //
 // Forward (one CTA per 128-query tile): the tile's key slots (global block 0 when include_cls, then the band
 // 4t-(left-1) .. 4t+3) are streamed four at a time through a 2-stage TMA ring; S = Q K^T double-buffered in TMEM
@@ -116,19 +115,9 @@ __device__ __forceinline__ float d_key_term(const DParams& p, int b, int key) {
   return p.kpm ? p.kpm[(int64_t)b * p.L + key] * kLog2e : 0.f;
 }
 
-// K-major operand (rows x 128 columns as two 16 KB halves): 16-column step ks = 0..7
-__device__ __forceinline__ uint64_t d_kdesc(uint32_t base, int ks) {
-  return make_smem_desc(base + (ks >> 2) * kDHalf + (ks & 3) * 32, 16, 1024, 128);
-}
-// MN-major B operand (K = 128 rows, N = 128 columns as two halves 16 KB apart): 16-row step k2 = 0..7
-__device__ __forceinline__ uint64_t d_mndesc(uint32_t base, int k2) {
-  return make_smem_desc(base + k2 * 16 * 128, kDHalf, 1024, 128);
-}
-
 // 128-row x 128-column tile -> two TMA boxes of 64 columns
 __device__ __forceinline__ void d_load_tile(uint8_t* dst, const CUtensorMap* map, uint64_t* bar, int row, int h, int b) {
-  tma_load_4d_w(dst, map, bar, 0, row, h, b);
-  tma_load_4d_w(dst + kDHalf, map, bar, 64, row, h, b);
+  load_rows<kDH>(dst, kDHalf, map, bar, row, h, b);
 }
 
 // 128 fp32 TMEM columns of one row -> 16-bit -> global row (16-byte stores)
@@ -232,7 +221,7 @@ attn_d128_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid
       const uint32_t k_addr = smem_u32(smem + S::OFF_K + s * kDTileB);
 #pragma unroll
       for (int ks = 0; ks < kDH / 16; ++ks)
-        mma_ss_w(tmem_base + 128 * s, d_kdesc(q_addr, ks), d_kdesc(k_addr, ks), idesc_s, ks > 0 ? 1u : 0u);
+        mma_ss_w(tmem_base + 128 * s, kmajor_desc(q_addr, ks, kDHalf), kmajor_desc(k_addr, ks, kDHalf), idesc_s, ks > 0 ? 1u : 0u);
       tc_commit_w(s_ready + s);
     };
     mbar_wait(q_full, 0);
@@ -246,7 +235,7 @@ attn_d128_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid
       const uint32_t v_addr = smem_u32(smem + S::OFF_V + s * kDTileB);
 #pragma unroll
       for (int k2 = 0; k2 < kTile / 16; ++k2)           // 16 keys per MMA: A = P (16-bit, 8 columns), B = V MN-major
-        mma_ts_w(tmem_base + COL_O, tmem_base + 128 * s + 8 * k2, d_mndesc(v_addr, k2), idesc_pv, (i > 0 || k2 > 0) ? 1u : 0u);
+        mma_ts_w(tmem_base + COL_O, tmem_base + 128 * s + 8 * k2, mnmajor_desc(v_addr, k2, kDHalf), idesc_pv, (i > 0 || k2 > 0) ? 1u : 0u);
       tc_commit_w(o_done);
       tc_commit_w(kv_free + s);
     }
@@ -464,8 +453,8 @@ attn_d128_bwd_dq_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       const uint32_t k_addr = smem_u32(smem + S::OFF_K + s * kDTileB), v_addr = smem_u32(smem + S::OFF_V + s * kDTileB);
 #pragma unroll
       for (int ks = 0; ks < kDH / 16; ++ks) {
-        mma_ss_w(tmem_base + S::COL_S, d_kdesc(q_addr, ks), d_kdesc(k_addr, ks), idesc_s, ks > 0 ? 1u : 0u);
-        mma_ss_w(tmem_base + S::COL_DP, d_kdesc(do_addr, ks), d_kdesc(v_addr, ks), idesc_s, ks > 0 ? 1u : 0u);
+        mma_ss_w(tmem_base + S::COL_S, kmajor_desc(q_addr, ks, kDHalf), kmajor_desc(k_addr, ks, kDHalf), idesc_s, ks > 0 ? 1u : 0u);
+        mma_ss_w(tmem_base + S::COL_DP, kmajor_desc(do_addr, ks, kDHalf), kmajor_desc(v_addr, ks, kDHalf), idesc_s, ks > 0 ? 1u : 0u);
       }
       tc_commit_w(s_ready);
     };
@@ -478,7 +467,7 @@ attn_d128_bwd_dq_sm100_kernel(const __grid_constant__ CUtensorMap tmQ, const __g
       const uint32_t k_addr = smem_u32(smem + S::OFF_K + s * kDTileB);
 #pragma unroll
       for (int k2 = 0; k2 < kTile / 16; ++k2)          // 16 keys per MMA: A = dS (16-bit, 8 columns), B = K MN-major
-        mma_ts_w(tmem_base + S::COL_DQ, tmem_base + S::COL_S + 8 * k2, d_mndesc(k_addr, k2), idesc_dq, (i > 0 || k2 > 0) ? 1u : 0u);
+        mma_ts_w(tmem_base + S::COL_DQ, tmem_base + S::COL_S + 8 * k2, mnmajor_desc(k_addr, k2, kDHalf), idesc_dq, (i > 0 || k2 > 0) ? 1u : 0u);
       if (p.cls && i == 0) {
         // dV_0^T (+)= dO^T [P_0 | dS_0], dK_0^T (+)= Q^T [P_0 | dS_0]: M = 128 head columns (two halves, MN-major),
         // K = 128 queries, N = 64
@@ -664,8 +653,8 @@ attn_d128_bwd_dkv_sm100_kernel(const __grid_constant__ CUtensorMap tmK, const __
       const uint32_t q_addr = smem_u32(smem + S::OFF_Q + s * kDTileB), do_addr = smem_u32(smem + S::OFF_DO + s * kDTileB);
 #pragma unroll
       for (int ks = 0; ks < kDH / 16; ++ks) {
-        mma_ss_w(tmem_base + S::COL_S, d_kdesc(k_addr, ks), d_kdesc(q_addr, ks), idesc_s, ks > 0 ? 1u : 0u);
-        mma_ss_w(tmem_base + S::COL_DP, d_kdesc(v_addr, ks), d_kdesc(do_addr, ks), idesc_s, ks > 0 ? 1u : 0u);
+        mma_ss_w(tmem_base + S::COL_S, kmajor_desc(k_addr, ks, kDHalf), kmajor_desc(q_addr, ks, kDHalf), idesc_s, ks > 0 ? 1u : 0u);
+        mma_ss_w(tmem_base + S::COL_DP, kmajor_desc(v_addr, ks, kDHalf), kmajor_desc(do_addr, ks, kDHalf), idesc_s, ks > 0 ? 1u : 0u);
       }
       tc_commit_w(s_ready);
     };
@@ -678,8 +667,8 @@ attn_d128_bwd_dkv_sm100_kernel(const __grid_constant__ CUtensorMap tmK, const __
       const uint32_t q_addr = smem_u32(smem + S::OFF_Q + s * kDTileB), do_addr = smem_u32(smem + S::OFF_DO + s * kDTileB);
 #pragma unroll
       for (int k2 = 0; k2 < kTile / 16; ++k2) {          // 16 queries per MMA; B = the dO / Q tile, MN-major
-        mma_ts_w(tmem_base + S::COL_DV, tmem_base + S::COL_S + 8 * k2, d_mndesc(do_addr, k2), idesc_o, (g > 0 || k2 > 0) ? 1u : 0u);
-        mma_ts_w(tmem_base + S::COL_DK, tmem_base + S::COL_DP + 8 * k2, d_mndesc(q_addr, k2), idesc_o, (g > 0 || k2 > 0) ? 1u : 0u);
+        mma_ts_w(tmem_base + S::COL_DV, tmem_base + S::COL_S + 8 * k2, mnmajor_desc(do_addr, k2, kDHalf), idesc_o, (g > 0 || k2 > 0) ? 1u : 0u);
+        mma_ts_w(tmem_base + S::COL_DK, tmem_base + S::COL_DP + 8 * k2, mnmajor_desc(q_addr, k2, kDHalf), idesc_o, (g > 0 || k2 > 0) ? 1u : 0u);
       }
       tc_commit_w(q_free + s);
       if (g + 1 < nc) issue_sdp(g + 1);

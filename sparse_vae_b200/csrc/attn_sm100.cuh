@@ -161,6 +161,28 @@ __device__ __forceinline__ void slot_exp_pack(const uint32_t (&v)[32], uint32_t 
 }
 
 
+// ---- 16-bit operand tiles of 64 or 128 columns in shared memory ---------------------------------------------------
+// A row of up to 64 elements is one SWIZZLE_128B atom.  A 128-element row is 256 bytes = two atoms, so a tile of
+// `rows` rows arrives as two TMA boxes of 64 columns (encode_tmap issues such boxes whenever Dh > 64), stored as two
+// halves of rows * 128 bytes (`half` below).  K-major operands (Q K^T) step through both halves; MN-major operands
+// (P V, dS K, P^T dO) span them with the descriptor's leading-byte offset = half.
+
+// K-major operand: 16-column step ks = 0 .. Dh/16 - 1
+__device__ __forceinline__ uint64_t kmajor_desc(uint32_t base, int ks, uint32_t half) {
+  return ptx::make_smem_desc(base + (ks >> 2) * half + (ks & 3) * 32, 16, 1024, 128);
+}
+// MN-major B operand (K = 16-row steps k2, N = Dh columns): the halves are `half` bytes apart
+__device__ __forceinline__ uint64_t mnmajor_desc(uint32_t base, int k2, uint32_t half) {
+  return ptx::make_smem_desc(base + k2 * 16 * 128, half, 1024, 128);
+}
+// `rows` rows starting at `row` of head h, sample b -> Dh / 64 boxes of 64 columns, `half` bytes apart
+template <int DH>
+__device__ __forceinline__ void load_rows(uint8_t* dst, uint32_t half, const CUtensorMap* map, uint64_t* bar, int row, int h,
+                                          int b) {
+#pragma unroll
+  for (int c = 0; c < DH / 64; ++c) ptx::tma_load_4d_w(dst + c * half, map, bar, 64 * c, row, h, b);
+}
+
 int encode_tmap(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int Dh, int L, int H, int B,
                 const int64_t stride[3], int box_rows);
 // 2-D map over a row-major 16-bit [rows, cols] matrix (row stride ld elements); box = 64 columns (one SWIZZLE_128B

@@ -233,7 +233,7 @@ static int launch_decode_dense(const void* q, const void* k, const void* v, cons
       decode_attn_dense_merge_kernel<T, DH><<<(unsigned)(B * H), DH, 0, st>>>(ws_max, ws_sum, ws_out, (T*)out, pos, H,   \
                                                                               cache_len, splits);                        \
   } while (0)
-  if (Dh == 64) SVAE_DEC_DENSE(64); else SVAE_DEC_DENSE(32);
+  if (Dh == 128) SVAE_DEC_DENSE(128); else if (Dh == 64) SVAE_DEC_DENSE(64); else SVAE_DEC_DENSE(32);
 #undef SVAE_DEC_DENSE
   SVAE_CUDA_CHECK(cudaGetLastError());
   return SVAE_OK;
@@ -244,7 +244,7 @@ static int launch_decode_dense(const void* q, const void* k, const void* v, cons
 using namespace svae;
 
 extern "C" int svae_decode_attn_dense_supported(int32_t head_dim, int32_t cache_len) {
-  return (head_dim == 32 || head_dim == 64) && cache_len >= 1 && cache_len <= kMaxCacheLen;
+  return (head_dim == 32 || head_dim == 64 || head_dim == 128) && cache_len >= 1 && cache_len <= kMaxCacheLen;
 }
 
 extern "C" size_t svae_decode_attn_dense_workspace_bytes(int32_t B, int32_t H, int32_t head_dim, int32_t cache_len) {
@@ -262,7 +262,7 @@ extern "C" int svae_decode_attn_dense(const void* q, const void* k, const void* 
   SVAE_REQUIRE(q && k && v && cos_table && sin_table && key_cache && value_cache && out && position, SVAE_ERR_INVALID,
                "svae_decode_attn_dense: null argument");
   SVAE_REQUIRE(svae_decode_attn_dense_supported(head_dim, cache_len), SVAE_ERR_UNSUPPORTED,
-               "svae_decode_attn_dense: head_dim %d / cache_len %d not supported (head_dim 32|64, cache_len 1..%d)",
+               "svae_decode_attn_dense: head_dim %d / cache_len %d not supported (head_dim 32|64|128, cache_len 1..%d)",
                head_dim, cache_len, kMaxCacheLen);
   SVAE_REQUIRE(B >= 0 && H > 0 && (int64_t)B * H <= INT32_MAX && table_rows > 0 &&
                    in_stride >= (int64_t)H * head_dim && in_stride % 8 == 0,
